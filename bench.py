@@ -22,6 +22,9 @@ Legs of one run, all over the same queries:
   e2e_device_abi   rtx_classify_batch with page-locked host buffers (the device boundary alone: H2D + kernels + D2H)
   roofline         the hit-count kernel, from per-launch CUDA events with the kernels serialised
   cpu_baseline     the CPU oracle port on the host cores over a bounded sample (rank 0, N = 1 only)
+
+--dump-outputs DIR writes the result arrays of the value leg's last timed step (c5: of its timed leg) as .npy files (dump_outputs): the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -202,6 +205,37 @@ def workload_queries(name, world, override=0):
     return base, per, scaling
 
 
+DUMP_BYTES = 60_000_000  # --dump-outputs: array bytes of one run, below 64 MB with the .npy headers
+DUMP_SEED = 20261020
+
+
+def dump_outputs(out, path, budget=DUMP_BYTES, first_query=0):
+    """Writes one step's ClassifyOutput (what a caller of the timed path receives) as float32 / float64 .npy files under `path`, so
+    that two builds can be compared output for output on the same inputs.  Every file is indexed by the queries in query.npy: all
+    queries when everything fits in `budget` bytes, otherwise the longest prefix of a fixed seeded permutation of the queries that
+    fits, in query order.  Per query: query (job-wide index), n_kmers, global_signal, n_results; per result line of those queries,
+    in query order: first_ref, n_levels, confidence [lines, max levels] (zero past n_levels) and local_signal."""
+    nq = len(out.n_kmers)
+    rb = out.result_begin.astype(np.int64)
+    n_lines = rb[1:] - rb[:-1]
+    n_lev = out.confidence.shape[1]
+    cost = (8 + 4 + 8 + 4) + n_lines * (8 + 4 + 8 * n_lev + 8)
+    order = np.random.default_rng(DUMP_SEED).permutation(nq)
+    q = np.sort(order[: int(np.searchsorted(np.cumsum(cost[order]), budget, side="right"))])
+    cnt = n_lines[q]
+    rows = np.repeat(rb[q] - (np.cumsum(cnt) - cnt), cnt) + np.arange(int(cnt.sum()))
+    lev = out.n_levels[rows]
+    conf = np.where(np.arange(n_lev)[None, :] < lev[:, None], out.confidence[rows], 0.0)
+    os.makedirs(path, exist_ok=True)
+    arrays = {"query": (q + first_query).astype(np.float64), "n_kmers": out.n_kmers[q].astype(np.float32),
+              "global_signal": out.global_signal[q].astype(np.float64), "n_results": cnt.astype(np.float32),
+              "first_ref": out.first_ref[rows].astype(np.float64), "n_levels": lev.astype(np.float32),
+              "confidence": conf.astype(np.float64), "local_signal": out.local_signal[rows].astype(np.float64)}
+    for k, a in arrays.items():
+        np.save(os.path.join(path, f"{k}.npy"), a)
+    print(f"--dump-outputs: {len(q)} of {nq} queries, {len(rows)} result lines -> {path}", file=sys.stderr)
+
+
 class CpuReference:
     """The reference algorithm (oracle port of raxtax.rs:14-97 with the chunked thread fan-out of main.rs:119-124) on host cores,
     over a bounded sample of the workload's queries."""
@@ -258,7 +292,13 @@ def main():
     ap.add_argument("--sub-batch", type=int, default=0, help="RTX_OPT_SUB_BATCH for the timed legs (0 = library default)")
     ap.add_argument("--pipeline", type=int, default=-1, help="RTX_OPT_PIPELINE for the timed legs (-1 = library default)")
     ap.add_argument("--chunk", type=int, default=0, help="chunk_size of rxh_raxtax in the e2e leg (0 = the driver's default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the timed leg returned in its last step to DIR/<name>.npy (see dump_outputs; DIR/rank<r>/ per rank when N > 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(min(args.warmup, 1), 1)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -341,8 +381,10 @@ def main():
     if name == "c5":
         from raxtax_b200 import bench_sharded
 
-        line = bench_sharded.run(args, rank, local_rank, world, barrier, max_over_ranks, load_workload, ClockSampler, measured_peaks, METRIC, UNIT)
+        line, out = bench_sharded.run(args, rank, local_rank, world, barrier, max_over_ranks, load_workload, ClockSampler, measured_peaks, METRIC, UNIT)
         if rank == 0:
+            if args.dump_outputs:  # the lines of every query end up on rank 0
+                dump_outputs(out, args.dump_outputs)
             emit(line)
         if world > 1:
             dist.destroy_process_group()
@@ -543,8 +585,8 @@ def main():
         from raxtax_b200 import bench_sharded
 
         n_sh = min(16384, q_per_rank)  # rank 0's slice starts at query 0: its unsharded results above are the expected lines
-        rec = bench_sharded.sharded_leg(ctx, tree, ds, n_sh, rank, world, max(1, min(args.steps, 5)), skip, dist, barrier, max_over_ranks,
-                                        expect=res if rank == 0 else None)
+        rec, _ = bench_sharded.sharded_leg(ctx, tree, ds, n_sh, rank, world, max(1, min(args.steps, 5)), skip, dist, barrier, max_over_ranks,
+                                           expect=res if rank == 0 else None)
         if rank == 0:
             assert rec["queries_differing_from_unsharded"] <= max(2, n_sh // 1000), f"reference-sharded run differs from the unsharded one on {rec['queries_differing_from_unsharded']} queries"
         line["sharded"] = rec
@@ -565,6 +607,11 @@ def main():
         ref.orc.set_flat_hist(True)
         s_flat = ref.run(n_small, cores, max(1, n_small // cores))
         line["cpu_baseline"]["std_map_variant"] = {"value": n_small / s_map, "flat_value_same_sample": n_small / s_flat, "sample": f"first {n_small} queries"}
+    if args.dump_outputs:  # res: the device-resident leg's last timed step, this rank's slice of the queries
+        if world == 1:
+            dump_outputs(res, args.dump_outputs)
+        else:
+            dump_outputs(res, os.path.join(args.dump_outputs, f"rank{rank}"), DUMP_BYTES // world, first_query=q0)
     if rank == 0:
         emit(line)
     ctx.close()

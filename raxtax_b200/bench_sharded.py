@@ -21,8 +21,9 @@ def broadcast_unique_id(dist, rank):
 
 
 def sharded_leg(ctx, tree, ds, n_queries, rank, world, steps, skip, dist, barrier, max_over_ranks, expect=None, sub_batch=0):
-    """Classifies the first n_queries queries of ds on `world` reference shards; returns the record for the bench line (rank 0) and
-    leaves ctx holding the sharded index.  expect = ClassifyOutput of the same queries from an unsharded context: compared line by line."""
+    """Classifies the first n_queries queries of ds on `world` reference shards; returns the record for the bench line (rank 0) and the
+    ClassifyOutput of the last timed step (the merged lines on rank 0), and leaves ctx holding the sharded index.  expect = ClassifyOutput
+    of the same queries from an unsharded context: compared line by line."""
     import torch
 
     N = tree.num_tips
@@ -94,11 +95,12 @@ def sharded_leg(ctx, tree, ds, n_queries, rank, world, steps, skip, dist, barrie
            "queries_differing_from_unsharded": n_diff,
            "identical_note": "compared line by line with rank 0's unsharded results of the same queries; flat-profile (K = 0) queries sit on exact "
                              "ties / rounding boundaries and may differ (DESIGN 2, tools/shard_diff.py)"}
-    return rec
+    return rec, out
 
 
 def run(args, rank, local_rank, world, barrier, max_over_ranks, load_workload, ClockSampler, measured_peaks, METRIC, UNIT):
-    """bench.py --workload c5: 8 M references (1 M per shard at 8 ranks), a bounded job of --queries queries (default 131 072)."""
+    """bench.py --workload c5: 8 M references (1 M per shard at 8 ranks), a bounded job of --queries queries (default 131 072).
+    Returns the bench line and the ClassifyOutput of the last timed step (every query's lines on rank 0)."""
     import torch
     import torch.distributed as dist
 
@@ -124,12 +126,12 @@ def run(args, rank, local_rank, world, barrier, max_over_ranks, load_workload, C
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            ctx.classify(off, codes, eo, eids)
+            out = ctx.classify(off, codes, eo, eids)
         secs = time.perf_counter() - t0
         rec = {"value": nq * args.steps / secs, "ms_per_step": 1e3 * secs / args.steps, "n_ranks": 1, "queries": nq, "through": "rtx_classify_batch, unsharded (one rank)",
                "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0, "gpu_launches": 0}
     else:
-        rec = sharded_leg(ctx, tree, ds, nq, rank, world, args.steps, False, dist, barrier, max_over_ranks, sub_batch=args.sub_batch)
+        rec, out = sharded_leg(ctx, tree, ds, nq, rank, world, args.steps, False, dist, barrier, max_over_ranks, sub_batch=args.sub_batch)
     clocks = sampler.stop()
     line = {"metric": METRIC, "value": rec["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": 2, "ms_per_step": rec["ms_per_step"],
             "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "u32 bit-planes/u16 counts/f64", "data": "synthetic",
@@ -140,4 +142,4 @@ def run(args, rank, local_rank, world, barrier, max_over_ranks, load_workload, C
                     "through": rec["through"]},
             "gpu_launches": rec["gpu_launches"], "sharded": rec}
     ctx.close()
-    return line
+    return line, out

@@ -1,15 +1,15 @@
 """Generates tests/golden/diptera_sample.fasta: the first 400 records of the reference repository's example data
 (example/diptera_queries.fasta, the only example file shipped; SURVEY.md 8(c) uses it as its own database).
-Run once in the build container where /root/reference exists; the GPU box only sees the committed sample."""
+Usage: make_diptera_sample.py <reference checkout>/example/diptera_queries.fasta; the tests read the committed sample only."""
 import os
+import sys
 
-SRC = "/root/reference/example/diptera_queries.fasta"
 DST = os.path.join(os.path.dirname(os.path.abspath(__file__)), "diptera_sample.fasta")
 N = 400
 
 if __name__ == "__main__":
     out, n = [], 0
-    for line in open(SRC):
+    for line in open(sys.argv[1]):
         if line.startswith(">"):
             n += 1
             if n > N:

@@ -22,9 +22,7 @@ def ctx():
 
 
 def _example_text():
-    src = "/root/reference/example/diptera_queries.fasta"  # present in the build container only
-    if os.path.exists(src):
-        return open(src).read()
+    """The reference repository's example/diptera_queries.fasta, stored whole (tests/golden/make_diptera_full.py)."""
     return gzip.open(os.path.join(GOLDEN, "diptera_queries.fasta.gz"), "rt").read()
 
 

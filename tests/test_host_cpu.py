@@ -353,6 +353,44 @@ def test_bench_strong_scaling_slices_cover_the_job_once():
     assert bench.workload_queries("c5", 8, 131072) == (131072, 131072, "strong")  # sharded references: every rank sees every query
 
 
+def test_bench_dump_outputs_bounded_and_reproducible(tmp_path):
+    """bench.py --dump-outputs: float32 / float64 arrays only, at most the byte budget, the same files for the same results, every query
+    while it all fits, and each dumped line the line of the query it is listed under."""
+    import bench
+
+    rng = np.random.default_rng(5)
+    nq, ML = 3000, 6
+    per_q = rng.integers(0, 9, nq)
+    rb = np.concatenate([[0], np.cumsum(per_q)]).astype(np.uint32)
+    n = int(rb[-1])
+    lev = rng.integers(1, ML + 1, n).astype(np.uint8)
+    out = capi.ClassifyOutput(rng.integers(0, 700, nq).astype(np.uint16), rb, rng.random(nq), rng.integers(0, 2**32 - 1, n, dtype=np.uint32),
+                              lev, rng.random((n, ML)), rng.random(n))
+
+    def load(d):
+        return {f[:-4]: np.load(os.path.join(d, f)) for f in sorted(os.listdir(d))}
+
+    bench.dump_outputs(out, str(tmp_path / "all"))
+    a = load(tmp_path / "all")
+    assert set(a) == {"query", "n_kmers", "global_signal", "n_results", "first_ref", "n_levels", "confidence", "local_signal"}
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert np.array_equal(a["query"], np.arange(nq)) and np.array_equal(a["first_ref"], out.first_ref.astype(np.float64))
+    assert np.array_equal(a["n_results"], per_q) and np.array_equal(a["n_kmers"], out.n_kmers)
+    lv = np.arange(ML)[None, :] < lev[:, None]
+    assert np.array_equal(a["confidence"][lv], out.confidence[lv]) and not a["confidence"][~lv].any()
+
+    budget = 100_000
+    for d in ("s1", "s2"):
+        bench.dump_outputs(out, str(tmp_path / d), budget, first_query=10_000)
+    s1, s2 = load(tmp_path / "s1"), load(tmp_path / "s2")
+    assert all(np.array_equal(s1[k], s2[k]) for k in s1)
+    assert 0 < len(s1["query"]) < nq and sum(v.nbytes for v in s1.values()) <= budget
+    q = s1["query"].astype(np.int64) - 10_000
+    assert np.all(np.diff(q) > 0) and np.array_equal(s1["n_results"], per_q[q])
+    rows = np.concatenate([np.arange(rb[i], rb[i + 1]) for i in q])
+    assert np.array_equal(s1["first_ref"], out.first_ref[rows]) and np.array_equal(s1["local_signal"], out.local_signal[rows])
+
+
 def test_chunk_plan_covers_every_query_once():
     """rxh_plan_chunks (the driver's par_chunks, raxtax.rs:35-39): consecutive, non-empty chunks that cover [0, n) exactly; an explicit
     chunk size is kept as given; the library's own choice starts and ends every context's share of the job with small chunks."""
