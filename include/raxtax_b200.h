@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define RTX_ABI_VERSION 3
+#define RTX_ABI_VERSION 4
 #define RTX_MAX_LEVELS 32 /* deepest lineage (comma-separated ranks) the device tree walk supports */
 #define RTX_MAX_RESULTS_PER_QUERY 256 /* >= the 200 lines a query can produce with the 0.01 cutoff */
 
@@ -52,19 +52,14 @@ typedef enum {
     RTX_OPT_SUB_BATCH = 2,      /* queries per device sub-batch (0 = auto) */
     RTX_OPT_KEEP_CSR = 3,       /* keep the CSR postings resident after building bit rows (needed for variant CSR) */
     RTX_OPT_PROFILE = 4,        /* record a CUDA event pair around every kernel launch (rtx_profile_get) */
-    RTX_OPT_HITCOUNT_TUNE = 5,  /* 0 = library default; 1..4 = row-load form of the query-group kernel (1: .v2 loads bypassing the L1,
-                                   2: .v2 through the L1 = default, 3: one-line loads through the L1, 4: one-line loads bypassing it);
-                                   >= 10 = single-query kernel geometry: V + 10*prefetch + 100*warps_per_cta */
-    RTX_OPT_HITCOUNT_MAX_TILES = 6, /* warp tiles (32*V words each) per CTA; fewer = more reference tile groups (L2 blocking); 0 = default */
+    RTX_OPT_HITCOUNT_MAX_TILES = 6, /* warp tiles (64 words each) per CTA; fewer = more reference tile groups (L2 blocking); 0 = default */
     RTX_OPT_HITCOUNT_GROUP = 7,     /* queries per CTA (one per warp) of the query-group bit-row kernel: 0 = library default (4; 16 when the
-                                       bit rows exceed 6 GB),
-                                       1 = single-query kernel (one warp per reference tile), 2..16 = group size, 101 = group kernel with 1 */
-    RTX_OPT_HITCOUNT_CHUNKS = 8,    /* row-id chunks the warps of a group cross in lockstep (block barrier per chunk) so that shared rows
-                                       hit the L1; 0 or 1 = no lockstep (default, fastest measured) */
+                                       bit rows reach 6 GB), 1 = single-query kernel (one query per CTA), 2..16 = group size; the size is
+                                       halved for long queries, and a sub-batch smaller than it runs the single-query kernel */
     RTX_OPT_WALK_VARIANT = 9,       /* tree walk: 0 = level-synchronous kernel + depth-first retry of overflowing queries (default),
-                                       1 = depth-first walker only, 2 = level-synchronous with 128-thread CTAs, 3 = level-synchronous
-                                       without the large-frontier paths (every child of a frontier node is evaluated), 4 = test hook:
-                                       those paths (mass-pruned search, arg-max over the kept segments) forced on every frontier */
+                                       1 = depth-first walker only, 3 = level-synchronous without the large-frontier paths (every child
+                                       of a frontier node is evaluated), 4 = test hook: those paths (mass-pruned search, arg-max over the
+                                       kept segments) forced on every frontier */
     RTX_OPT_PIPELINE = 11,          /* 1: batches of >= 4096 queries are cut into >= 4 sub-batches and hit counting of sub-batch i+1 overlaps
                                        probabilities / prefix sums / tree walk of sub-batch i on a second, higher-priority stream;
                                        0 (default) = serial: on B200 the overlap only recovers what the shorter launches lose */

@@ -21,8 +21,8 @@ u8p, u16p, u32p, u64p, f64p = (C.POINTER(t) for t in (C.c_uint8, C.c_uint16, C.c
 RTX_OK, RTX_ERR_INVALID, RTX_ERR_CUDA, RTX_ERR_NO_DEVICE, RTX_ERR_NO_INDEX, RTX_ERR_UNSUPPORTED, RTX_ERR_ASSERT = 0, -1, -2, -3, -4, -5, -6
 RTX_SKIP_EXACT_MATCHES, RTX_RAW_CONFIDENCE = 1, 2
 RTX_HITCOUNT_BITROWS, RTX_HITCOUNT_CSR = 0, 1
-RTX_OPT_HITCOUNT_VARIANT, RTX_OPT_SUB_BATCH, RTX_OPT_KEEP_CSR, RTX_OPT_PROFILE, RTX_OPT_HITCOUNT_TUNE, RTX_OPT_HITCOUNT_MAX_TILES = 1, 2, 3, 4, 5, 6
-RTX_OPT_HITCOUNT_GROUP, RTX_OPT_HITCOUNT_CHUNKS, RTX_OPT_WALK_VARIANT, RTX_OPT_WALK_LOG_CAP, RTX_OPT_PIPELINE = 7, 8, 9, 10, 11
+RTX_OPT_HITCOUNT_VARIANT, RTX_OPT_SUB_BATCH, RTX_OPT_KEEP_CSR, RTX_OPT_PROFILE, RTX_OPT_HITCOUNT_MAX_TILES = 1, 2, 3, 4, 6
+RTX_OPT_HITCOUNT_GROUP, RTX_OPT_WALK_VARIANT, RTX_OPT_WALK_LOG_CAP, RTX_OPT_PIPELINE = 7, 9, 10, 11
 KERNEL_NAMES = ["kmers", "hitcount", "fixup", "prob", "index", "walk", "prefix", "allreduce", "allgather", "shard", "gather"]
 
 # every symbol include/raxtax_b200.h declares

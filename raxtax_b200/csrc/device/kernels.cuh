@@ -20,13 +20,6 @@ namespace rtx {
 // =========================================================================================================
 // small helpers
 // =========================================================================================================
-__device__ __forceinline__ uint4 ldg_stream(const uint4* p) {
-    uint4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
-                 : "l"(p));
-    return r;
-}
 __device__ __forceinline__ uint2 ldg_stream(const uint2* p) {
     uint2 r;
     asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];" : "=r"(r.x), "=r"(r.y) : "l"(p));
@@ -233,15 +226,15 @@ __global__ void __launch_bounds__(kKmerThreads) kmers_kernel(IndexView ix, Batch
 // =========================================================================================================
 // K2: hit counting by positional popcount.
 //
-// count[r] = |kmers(q) ∩ kmers(ref r)| = column sum over the query's bit rows.  Each lane owns V consecutive
-// 32-bit words of the row (32·V references) and keeps the column sums bit-sliced: plane p of a word holds bit p
+// count[r] = |kmers(q) ∩ kmers(ref r)| = column sum over the query's bit rows.  Each lane owns kLaneWords consecutive
+// 32-bit words of the row (64 references) and keeps the column sums bit-sliced: plane p of a word holds bit p
 // of the 32 counters.  16 rows are folded per step with a carry-save adder tree (15 full adders = 30 LOP3)
 // whose single weight-16 carry ripples into the high planes.  The epilogue transposes the planes into 32 u16
 // counters with a 16x16 bit-matrix transpose done on both half-words at once, stores them and feeds the
 // shared-memory histogram.
 // =========================================================================================================
 constexpr int kHitThreads = 256;
-constexpr int kHitWarps = kHitThreads / 32;
+constexpr int kLaneWords = 2;      // words of a row per lane: one 8-byte load per row, a warp tile is 64 words = 2048 references
 constexpr int kRowListCap = 4096;  // row ids staged in shared memory per chunk
 
 __device__ __forceinline__ void csa(u32& s, u32& c, u32 a, u32 b, u32 d) {
@@ -272,10 +265,6 @@ __device__ __forceinline__ void ripple(u32 (&pl)[NP], u32 e) {
         pl[p] ^= e;
         e = t;
     }
-}
-template <int NP>
-__device__ __forceinline__ void add16(u32 (&pl)[NP], const u32 (&x)[16]) {
-    ripple<NP, 4>(pl, add16_carry<NP>(pl, x));
 }
 // two weight-16 carries: one full adder into plane 4, then a single ripple from plane 5
 template <int NP>
@@ -312,23 +301,12 @@ __device__ __forceinline__ void planes_to_counts(const u32 (&pl)[NP], u32 (&out)
     }
 }
 
-template <int V>
-struct RowVec;
-template <>
-struct RowVec<2> {
-    typedef uint2 T;
-};
-template <>
-struct RowVec<4> {
-    typedef uint4 T;
-};
 __device__ __forceinline__ u32 vec_get(const uint2& v, int i) { return i == 0 ? v.x : v.y; }
-__device__ __forceinline__ u32 vec_get(const uint4& v, int i) { return i == 0 ? v.x : i == 1 ? v.y : i == 2 ? v.z : v.w; }
 
 // grid: x = query within the sub-batch, y = tile group.  block: 32 * nwarps threads (nwarps chosen by the host so that
 // the tiles of a CTA divide evenly over its warps).
 // dynamic shared memory: u32 srow[kRowListCap] + u32 shist[hstride]
-// PF = software prefetch: the next 16 rows are requested before the current 16 are folded (register double buffer).
+// The next 16 rows are requested before the current 16 are folded (register double buffer).
 // address of a row's slice: one IMAD.WIDE on the fma pipe (the compiler's own choice, IMAD.WIDE + two LEAs, put a third of
 // the inner loop's alu-pipe work into address arithmetic; LOP3 shares that pipe at half rate)
 __device__ __forceinline__ const void* row_ptr(const u32* __restrict__ colbase, u32 rid, u32 row_bytes) {
@@ -347,58 +325,41 @@ __device__ __forceinline__ void row_ids16(u32 (&r)[16], const u32* __restrict__ 
         r[4 * i] = t.x, r[4 * i + 1] = t.y, r[4 * i + 2] = t.z, r[4 * i + 3] = t.w;
     }
 }
-template <int V, typename vec_t>
-__device__ __forceinline__ void load16(vec_t (&x)[16], const u32* __restrict__ colbase, const u32* __restrict__ srow, u32 j, u32 row_bytes) {
+__device__ __forceinline__ void load16(uint2 (&x)[16], const u32* __restrict__ colbase, const u32* __restrict__ srow, u32 j, u32 row_bytes) {
     u32 r[16];
     row_ids16(r, srow, j);
 #pragma unroll
-    for (int i = 0; i < 16; ++i) x[i] = ldg_stream(reinterpret_cast<const vec_t*>(row_ptr(colbase, r[i], row_bytes)));
-}
-template <int V, int NP, typename vec_t>
-__device__ __forceinline__ void fold16(u32 (&pl)[V][NP], const vec_t (&x)[16]) {
-#pragma unroll
-    for (int v = 0; v < V; ++v) {
-        u32 xv[16];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) xv[i] = vec_get(x[i], v);
-        add16<NP>(pl[v], xv);
-    }
+    for (int i = 0; i < 16; ++i) x[i] = ldg_stream(reinterpret_cast<const uint2*>(row_ptr(colbase, r[i], row_bytes)));
 }
 
-template <int V, int NP, typename vec_t>
-__device__ __forceinline__ void fold16_carry(u32 (&pl)[V][NP], const vec_t (&x)[16], u32 (&e)[V]) {
+template <int NP>
+__device__ __forceinline__ void fold16_carry(u32 (&pl)[kLaneWords][NP], const uint2 (&x)[16], u32 (&e)[kLaneWords]) {
 #pragma unroll
-    for (int v = 0; v < V; ++v) {
+    for (int v = 0; v < kLaneWords; ++v) {
         u32 xv[16];
 #pragma unroll
         for (int i = 0; i < 16; ++i) xv[i] = vec_get(x[i], v);
         e[v] = add16_carry<NP>(pl[v], xv);
     }
 }
-template <int V, int NP>
-__device__ __forceinline__ void merge_carries_v(u32 (&pl)[V][NP], const u32 (&ea)[V], const u32 (&eb)[V]) {
+template <int NP>
+__device__ __forceinline__ void merge_carries_v(u32 (&pl)[kLaneWords][NP], const u32 (&ea)[kLaneWords], const u32 (&eb)[kLaneWords]) {
 #pragma unroll
-    for (int v = 0; v < V; ++v) merge_carries<NP>(pl[v], ea[v], eb[v]);
+    for (int v = 0; v < kLaneWords; ++v) merge_carries<NP>(pl[v], ea[v], eb[v]);
 }
 
 // The count vectors (2 * N bytes per query, tens of GB per launch) are written once and read back much later, if at all: streaming
 // stores (evict-first) keep them from pushing the L2-blocked slice of the bit matrix out of the L2.
-__device__ __forceinline__ void store_counts(uint4* p, const uint4& v) {
-#ifdef RTX_COUNTS_PLAIN_STORE
-    *p = v;
-#else
-    __stcs(p, v);
-#endif
-}
+__device__ __forceinline__ void store_counts(uint4* p, const uint4& v) { __stcs(p, v); }
 
-template <int V, int NP, bool PF>
+template <int NP>
 __global__ void __launch_bounds__(kHitThreads)
     hitcount_bitrows_kernel(IndexView ix, BatchView b, u16* __restrict__ counts, int q_base, int tiles_per_cta, int n_tiles, int hist_global) {
+    constexpr int V = kLaneWords;
     extern __shared__ __align__(16) u32 hsm[];
     u32* srow = hsm;
     // hist_global: queries with tens of thousands of 8-mers, whose histogram does not fit shared memory: bins are bumped in global memory
     u32* shist = hist_global ? b.hist + (size_t)(q_base + blockIdx.x) * b.hstride : hsm + kRowListCap;
-    typedef typename RowVec<V>::T vec_t;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int nthreads = blockDim.x, nwarps = nthreads >> 5;
     const int ql = blockIdx.x;
@@ -439,28 +400,20 @@ __global__ void __launch_bounds__(kHitThreads)
             }
             if (active) {
                 const u32* __restrict__ colbase = ix.bitrows + word0;
-                if (PF) {
-                    vec_t xa[16], xb[16];
-                    load16<V>(xa, colbase, srow, 0, row_bytes);
-                    for (u32 j = 0; j < cn; j += 32) {
-                        const bool has_b = j + 16 < cn;
-                        u32 ea[V], eb[V];
-                        if (has_b) load16<V>(xb, colbase, srow, j + 16, row_bytes);
-                        fold16_carry<V, NP>(pl, xa, ea);
-                        if (j + 32 < cn) load16<V>(xa, colbase, srow, j + 32, row_bytes);
-                        if (has_b) fold16_carry<V, NP>(pl, xb, eb);
-                        else {
+                uint2 xa[16], xb[16];
+                load16(xa, colbase, srow, 0, row_bytes);
+                for (u32 j = 0; j < cn; j += 32) {
+                    const bool has_b = j + 16 < cn;
+                    u32 ea[V], eb[V];
+                    if (has_b) load16(xb, colbase, srow, j + 16, row_bytes);
+                    fold16_carry<NP>(pl, xa, ea);
+                    if (j + 32 < cn) load16(xa, colbase, srow, j + 32, row_bytes);
+                    if (has_b) fold16_carry<NP>(pl, xb, eb);
+                    else {
 #pragma unroll
-                            for (int v = 0; v < V; ++v) eb[v] = 0;
-                        }
-                        merge_carries_v<V, NP>(pl, ea, eb);
+                        for (int v = 0; v < V; ++v) eb[v] = 0;
                     }
-                } else {
-                    for (u32 j = 0; j < cn; j += 16) {
-                        vec_t x[16];
-                        load16<V>(x, colbase, srow, j, row_bytes);
-                        fold16<V, NP>(pl, x);
-                    }
+                    merge_carries_v<NP>(pl, ea, eb);
                 }
             }
         }
@@ -502,70 +455,38 @@ __global__ void __launch_bounds__(kHitThreads)
 // K2 (query-group form): the single-query kernel above sits exactly on the L2 -> SM bandwidth cap (every bit row of every
 // query is fetched from L2 once per reference tile: 82 GB per 10 k queries on C2 = 12.4 TB/s).  Queries of one batch share
 // rows (two COI queries have ~22 % of their 8-mers in common; the union of 16 queries' rows is ~half the sum), so here a
-// CTA carries G queries -- one per warp -- over the SAME reference tile and keeps them in lockstep over the row-id space:
-// the sorted row lists are cut at common row-id boundaries ("chunks") and a block barrier separates the chunks, so that a
-// row wanted by several warps is requested within one chunk's time window and all but the first request hit the L1
-// (plain ld.global.nc, L1-allocating; one chunk's union of rows is sized to fit the L1 carve-out).
+// CTA carries G queries -- one per warp -- over the SAME reference tile.  The row loads allocate in the L1 (plain
+// ld.global.nc), so that a row that another warp of the CTA has fetched shortly before hits there instead of going to the L2.
+// The warps run independently, with no block barrier: keeping them in step over the row-id space raises the L1 hit rate but
+// the barriers cost more than the hits save (DESIGN.md §4, K2).
 // grid: x = query group (fastest: L2 blocking over reference tile groups as before), y = tile group.
-// dynamic smem: u32 srow[G][kstride] | u32 shist[G][hstride] | u16 cpos[G][n_chunks]
+// dynamic smem: u32 srow[G][kstride] | u32 shist[G][hstride]
 // =========================================================================================================
 __device__ __forceinline__ uint2 ldg_l1(const uint2* p) {
     uint2 r;
     asm volatile("ld.global.nc.v2.u32 {%0,%1}, [%2];" : "=r"(r.x), "=r"(r.y) : "l"(p));
     return r;
 }
-__device__ __forceinline__ uint4 ldg_l1(const uint4* p) {
-    uint4 r;
-    asm volatile("ld.global.nc.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-    return r;
-}
-__device__ __forceinline__ u32 ldg_l1_u32(const u32* p) {
-    u32 r;
-    asm volatile("ld.global.nc.u32 %0, [%1];" : "=r"(r) : "l"(p));
-    return r;
-}
-__device__ __forceinline__ u32 ldg_stream_u32(const u32* p) {
-    u32 r;
-    asm volatile("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(r) : "l"(p));
-    return r;
-}
-// SPLIT: a lane's two words of a row are NOT neighbours (words l and l + 32 of the warp's 64-word slice): every load instruction of
-// the warp then covers exactly one 128-byte line.  A warp-wide LDG that touches two lines (the .v2 form: 256 bytes per warp) is
-// replayed per line at ~2.07 cycles each in the L1's data stage, two one-line LDGs cost ~1.0 cycle each (B300_MICROARCH.md, "L1tex
-// wavefront queue") -- the kernel sat at 59 B/clk/SM of row slices, the two-line rate, with that unit 80 % busy.
-template <int V, bool L1A, bool SPLIT, typename vec_t>
-__device__ __forceinline__ void load16_l1(vec_t (&x)[16], const u32* __restrict__ colbase, const u32* __restrict__ srow, u32 j, u32 row_bytes) {
+__device__ __forceinline__ void load16_l1(uint2 (&x)[16], const u32* __restrict__ colbase, const u32* __restrict__ srow, u32 j) {
     u32 r[16];
     row_ids16(r, srow, j);
 #pragma unroll
-    for (int i = 0; i < 16; ++i) {
-        if constexpr (SPLIT && V == 2) {
-            const u32* p = reinterpret_cast<const u32*>(reinterpret_cast<const char*>(colbase) + (u64)r[i] * 512u);
-            x[i].x = L1A ? ldg_l1_u32(p) : ldg_stream_u32(p);
-            x[i].y = L1A ? ldg_l1_u32(p + 32) : ldg_stream_u32(p + 32);
-        } else {
-            const vec_t* p = reinterpret_cast<const vec_t*>(reinterpret_cast<const char*>(colbase) + (u64)r[i] * 512u);
-            x[i] = L1A ? ldg_l1(p) : ldg_stream(p);
-        }
-    }
+    for (int i = 0; i < 16; ++i) x[i] = ldg_l1(reinterpret_cast<const uint2*>(reinterpret_cast<const char*>(colbase) + (u64)r[i] * 512u));
 }
 
 constexpr int kHitGroupMaxThreads = 512;
 
-// LOCKSTEP = false drops the chunk bookkeeping and every block barrier (the warps of a CTA then only share the launch).
 // (A 96-register build, 5 CTAs x 4 warps per SM instead of 4 x 4, spills and measured 6 % slower.)
-// L1A: row loads allocate in the L1 (rows shared by the warps of a CTA may hit) or bypass it (no fill wavefronts on the L1 data pipe)
-template <int V, int NP, bool LOCKSTEP, int MAX_THREADS, int CTAS_PER_SM, bool L1A = true, bool SPLIT = false>
-__global__ void __launch_bounds__(MAX_THREADS, CTAS_PER_SM)
+template <int NP>
+__global__ void __launch_bounds__(kHitGroupMaxThreads, 1)
     hitcount_group_kernel(IndexView ix, BatchView b, u16* __restrict__ counts, int q_base, int q_count, int tiles_per_cta, int n_tiles,
-                          u32 chunk_rows, int n_chunks, u16* __restrict__ segmax, size_t segmax_stride) {
+                          u16* __restrict__ segmax, size_t segmax_stride) {
+    constexpr int V = kLaneWords;
     extern __shared__ __align__(16) u32 hsm[];
-    typedef typename RowVec<V>::T vec_t;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int G = blockDim.x >> 5;
     u32* srow = hsm + (size_t)warp * b.kstride;
     u32* shist = hsm + (size_t)G * b.kstride + (size_t)warp * b.hstride;
-    u16* cpos = reinterpret_cast<u16*>(hsm + (size_t)G * (b.kstride + b.hstride)) + (size_t)warp * n_chunks;
     const int ql = blockIdx.x * G + warp;
     const bool valid = ql < q_count;
     const int q = q_base + (valid ? ql : 0);
@@ -578,58 +499,32 @@ __global__ void __launch_bounds__(MAX_THREADS, CTAS_PER_SM)
     for (u32 i = lane; i < n; i += 32) srow[i] = qrows[i] * row_units;
     for (u32 i = lane; i < nbins; i += 32) shist[i] = 0;
     __syncwarp();
-    // chunk c holds the rows with id in [c * chunk_rows, (c + 1) * chunk_rows); cpos[c] = list position where it ends
-    for (int c = lane; LOCKSTEP && c < n_chunks; c += 32) {
-        u32 lo = 0, hi = n;
-        if (c < n_chunks - 1) {
-            const u32 bound = (u32)(c + 1) * chunk_rows * row_units;  // the staged list holds scaled ids
-            while (lo < hi) {
-                const u32 mid = (lo + hi) >> 1;
-                const u32 x = srow[mid];
-                if (x != 0u && x < bound) lo = mid + 1;  // the padding rows (id 0) sit at the end of the ascending list
-                else hi = mid;
-            }
-        } else lo = n;
-        cpos[c] = (u16)lo;
-    }
-    __syncwarp();
 
     const int tile_begin = blockIdx.y * tiles_per_cta;
     const int tile_end = min(n_tiles, tile_begin + tiles_per_cta);
-    const u32 row_bytes = ix.row_words * 4u;
     u16* __restrict__ qcounts = counts + (size_t)ql * ix.n_pad;
-    constexpr int kWordStep = SPLIT ? 32 : 1;  // distance between a lane's words
     for (int tile = tile_begin; tile < tile_end; ++tile) {
-        const u32 word0 = (u32)tile * (32 * V) + (SPLIT ? lane : lane * V);
+        const u32 word0 = (u32)tile * (32 * V) + lane * V;
         const u32* __restrict__ colbase = ix.bitrows + word0;
         u32 pl[V][NP];
 #pragma unroll
         for (int v = 0; v < V; ++v)
 #pragma unroll
             for (int p = 0; p < NP; ++p) pl[v][p] = 0;
-        int c = 0;
-        vec_t xa[16], xb[16];
-        if (n) load16_l1<V, L1A, SPLIT>(xa, colbase, srow, 0, row_bytes);
+        uint2 xa[16], xb[16];
+        if (n) load16_l1(xa, colbase, srow, 0);
         for (u32 j = 0; j < n; j += 32) {
-            while (LOCKSTEP && c < n_chunks && j >= (u32)cpos[c]) {  // this warp is done with chunk c: wait for the others
-                __syncthreads();
-                ++c;
-            }
             const bool has_b = j + 16 < n;
             u32 ea[V], eb[V];
-            if (has_b) load16_l1<V, L1A, SPLIT>(xb, colbase, srow, j + 16, row_bytes);
-            fold16_carry<V, NP>(pl, xa, ea);
-            if (j + 32 < n) load16_l1<V, L1A, SPLIT>(xa, colbase, srow, j + 32, row_bytes);
-            if (has_b) fold16_carry<V, NP>(pl, xb, eb);
+            if (has_b) load16_l1(xb, colbase, srow, j + 16);
+            fold16_carry<NP>(pl, xa, ea);
+            if (j + 32 < n) load16_l1(xa, colbase, srow, j + 32);
+            if (has_b) fold16_carry<NP>(pl, xb, eb);
             else {
 #pragma unroll
                 for (int v = 0; v < V; ++v) eb[v] = 0;
             }
-            merge_carries_v<V, NP>(pl, ea, eb);
-        }
-        while (LOCKSTEP && c < n_chunks) {
-            __syncthreads();
-            ++c;
+            merge_carries_v<NP>(pl, ea, eb);
         }
         if (valid) {
             u32 lane_max = 0;  // largest count among this lane's 32 * V references, in both half-words
@@ -641,14 +536,7 @@ __global__ void __launch_bounds__(MAX_THREADS, CTAS_PER_SM)
 #pragma unroll
                 for (int i = 0; i < 16; ++i) word_max = __vmaxu2(word_max, out[i]);
                 lane_max = __vmaxu2(lane_max, word_max);
-                if (SPLIT && segmax != nullptr) {
-                    // word lane + 32 v of the tile: 16 lanes share a 512-reference segment, segment (tile * 64 + 32 v + lane) / 16
-                    u32 m = max(word_max & 0xFFFFu, word_max >> 16);
-#pragma unroll
-                    for (int o = 1; o < 16; o <<= 1) m = max(m, __shfl_xor_sync(kFullMask, m, o));
-                    if ((lane & 15) == 0) segmax[(size_t)ql * segmax_stride + (size_t)tile * 4 + 2 * v + (lane >> 4)] = (u16)m;
-                }
-                const u64 ref0 = (u64)(word0 + v * kWordStep) * 32;
+                const u64 ref0 = (u64)(word0 + v) * 32;
                 uint4* dst = reinterpret_cast<uint4*>(qcounts + ref0);
 #pragma unroll
                 for (int i = 0; i < 4; ++i) store_counts(dst + i, make_uint4(out[4 * i], out[4 * i + 1], out[4 * i + 2], out[4 * i + 3]));
@@ -668,7 +556,7 @@ __global__ void __launch_bounds__(MAX_THREADS, CTAS_PER_SM)
             }
             // largest count per 512-reference prefix segment (32 * V = 64 references per lane: 8 lanes per segment), so that K4 can
             // drop a segment below m_min without reading its counts (padding references count 0 and never raise the maximum)
-            if (!SPLIT && segmax != nullptr) {
+            if (segmax != nullptr) {
                 u32 m = max(lane_max & 0xFFFFu, lane_max >> 16);
                 constexpr int kLanesPerSeg = 512 / (32 * V);
 #pragma unroll
@@ -2138,7 +2026,8 @@ constexpr u32 kBfsSmallNode = 48;                     // arg-max pairs: a node w
 constexpr u32 kBfsLeaf = 64;                          // search: runs this short are evaluated child by child
 constexpr u32 kBfsQueue = 256;                        // search: runs in flight per round
 constexpr double kBfsMassFloor = 0.004999;            // a child is significant from 0.005 on; the margin covers the rounding of the sums
-constexpr int kBfsThreadsDefault = 256;  // CTA size of lineage_bfs_kernel (template parameter: RTX_OPT_WALK_VARIANT 2 runs 128)
+constexpr int kBfsThreads = 256;  // CTA size of lineage_bfs_kernel
+constexpr int kBfsWarps = kBfsThreads / 32;
 constexpr u32 kBfsPtabSmemMax = 16384;   // the query's P(m) table is staged behind BfsSmem when it fits (K <= 2047), see bfs_ptab_smem
 __host__ __device__ inline size_t bfs_ptab_smem(u32 hstride) { return (size_t)hstride * 8 <= kBfsPtabSmemMax ? (size_t)hstride * 8 : 0; }
 // ... and so is its skip bitmap (one bit per 512-reference segment)
@@ -2252,7 +2141,6 @@ __device__ __forceinline__ u32 bfs_lower_bound(const u32* __restrict__ a, u32 n,
 // the flattened child list.  Runs of one node are clipped against their predecessor, so no child appears twice.  Children are sorted
 // and disjoint (tree.rs:77-107), their [lo, lo + size) are read from the node records.  Block-wide (four barriers); returns P.
 // (shard_begin: first reference of this shard -- segments count local references; skip_strad as in bfs_child_offsets)
-template <int kBfsThreads>
 __device__ u32 bfs_build_pairs(const BfsSmem& w, const NodeRec* __restrict__ recs, u32 n, u32 range_begin, const u16* __restrict__ list,
                                u32 n_kept, int tid, u32 shard_begin, bool skip_strad, u32 small_node) {
     const int lane = tid & 31, warp = tid >> 5;
@@ -2351,10 +2239,9 @@ __device__ __forceinline__ double bfs_child_prefix(const NodeRec* __restrict__ r
 // SH (reference-sharded walk): the prefixes only know this shard's references.  Of a large node's children those that touch the shard
 // [sh_lo, sh_hi) are found by binary search; the first and the last of them may straddle a cut (their confidence comes from the
 // combined records) and are always looked at, the ones in between lie inside the shard and are searched by mass.
-template <int kBfsThreads, bool SH>
+template <bool SH>
 __device__ u32 bfs_search_pairs(const BfsSmem& w, const NodeRec* __restrict__ recs, const MassView& mv, u32 n, u32 range_begin, u32* ctr, int tid,
                                 u64 sh_lo, u64 sh_hi, u32 leaf_len) {
-    constexpr int kBfsWarps = kBfsThreads / 32;
     const int lane = tid & 31, warp = tid >> 5;
     const u32 lt_mask = (1u << lane) - 1u;
     if (tid < 4) ctr[tid] = 0u;
@@ -2498,11 +2385,10 @@ __device__ u32 bfs_search_pairs(const BfsSmem& w, const NodeRec* __restrict__ re
 // from the combined records, a child inside another shard is left to its owner; a straddling node learns from the combined flags whether
 // it has a significant child / whether a line is pushed below it, and is reported by the rank that holds its first reference; a fallback
 // chain follows the combined best child through straddling nodes and ends where it leaves the shard.
-template <int kBfsThreads, bool SH>
+template <bool SH>
 __global__ void __launch_bounds__(kBfsThreads)  // (a 6-CTA/SM bound, 40 registers with small spills, measured the same 0.89 ms)
     lineage_bfs_kernel(IndexView ix, const NodeRec* __restrict__ recs, BatchView b, ResultPool pool, ProbScratch sc, ShardView sv, int q_base,
                        int q_count, u32 entry_cap, int sparse) {
-    constexpr int kBfsWarps = kBfsThreads / 32;
     extern __shared__ __align__(16) unsigned char bsm_raw[];
     __shared__ u32 s_log_n, s_n_res, s_n_fb, s_n_next, s_retry, s_retry_cls;  // s_retry_cls: raised while sorting a frontier (see the level loop)
     __shared__ u32 s_n_kept;  // kept segments of a sparse query, 0 = the arg-max looks at every child
@@ -2643,7 +2529,7 @@ __global__ void __launch_bounds__(kBfsThreads)  // (a 6-CTA/SM bound, 40 registe
             u32 total = w.fr_off[nf], n_own = nf;
             const bool pairs = sparse != 0 && total >= pair_min;  // block-uniform
             if (pairs) {
-                n_own = bfs_search_pairs<kBfsThreads, SH>(w, recs, mv, nf, lvl_begin, s_ctr, tid, sh_lo, sh_hi, leaf_len);
+                n_own = bfs_search_pairs<SH>(w, recs, mv, nf, lvl_begin, s_ctr, tid, sh_lo, sh_hi, leaf_len);
                 if (n_own == ~0u) {  // (every thread sees the same return value)
                     if (tid == 0) s_retry = 1;
                     break;
@@ -2743,7 +2629,7 @@ __global__ void __launch_bounds__(kBfsThreads)  // (a 6-CTA/SM bound, 40 registe
             u32 total = w.fr_off[n_ch], n_own = n_ch;
             const bool pairs = n_kept != 0 && total >= pair_min;  // block-uniform
             if (pairs) {
-                n_own = bfs_build_pairs<kBfsThreads>(w, recs, n_ch, 0, cur, n_kept, tid, (u32)sh_lo, SH, small_node);
+                n_own = bfs_build_pairs(w, recs, n_ch, 0, cur, n_kept, tid, (u32)sh_lo, SH, small_node);
                 total = w.fr_off[n_own];
             }
             for (u32 i = tid; i < n_ch; i += kBfsThreads) {

@@ -83,12 +83,10 @@ struct rtx_ctx : BatchState {
     int64_t sub_batch_opt = 0;
     bool keep_csr = false;
     bool profile = false;
-    int hit_tune = 0;
     int hit_max_tiles = 0;
     int walk_variant = 0;  // RTX_OPT_WALK_VARIANT: 0 level-synchronous (+ depth-first retry), 1 depth-first only
     int walk_log_cap = 0;  // RTX_OPT_WALK_LOG_CAP
     int hit_group = 0;   // RTX_OPT_HITCOUNT_GROUP
-    int hit_chunks = 0;  // RTX_OPT_HITCOUNT_CHUNKS
     // index
     bool has_index = false;
     IndexView ix{};
@@ -373,7 +371,7 @@ RTX_API int rtx_ctx_set_option(rtx_ctx* ctx, int option, int64_t value) {
             ctx->pipeline_opt = value != 0;
             return RTX_OK;
         case RTX_OPT_WALK_VARIANT:
-            REQUIRE(value >= 0 && value <= 4, "unknown walk variant");  // 2: 128-thread CTAs, 3: without the large-frontier paths, 4: with them forced
+            REQUIRE(value >= 0 && value <= 4 && value != 2, "unknown walk variant");  // 3: without the large-frontier paths, 4: with them forced
             ctx->walk_variant = (int)value;
             return RTX_OK;
         case RTX_OPT_WALK_LOG_CAP:
@@ -381,17 +379,8 @@ RTX_API int rtx_ctx_set_option(rtx_ctx* ctx, int option, int64_t value) {
             ctx->walk_log_cap = (int)value;
             return RTX_OK;
         case RTX_OPT_HITCOUNT_GROUP:
-            REQUIRE((value >= 0 && value <= kHitGroupMaxThreads / 32) || value == 101, "bad query group size");  // 101: group kernel with one query per CTA (experiments)
+            REQUIRE(value >= 0 && value <= kHitGroupMaxThreads / 32, "bad query group size");
             ctx->hit_group = (int)value;
-            return RTX_OK;
-        case RTX_OPT_HITCOUNT_CHUNKS:
-            REQUIRE(value >= 0 && value <= 4096, "bad chunk count");
-            ctx->hit_chunks = (int)value;
-            return RTX_OK;
-        case RTX_OPT_HITCOUNT_TUNE:
-            REQUIRE((value >= 0 && value <= 4) || (value >= 10 && value < 1000 && (value % 10 == 0 || value % 10 == 2 || value % 10 == 4)),
-                    "bad hit-count tuning word");  // 1..4: load form of the query-group kernel (launch_hitcount_group); >= 10: single-query kernel geometry
-            ctx->hit_tune = (int)value;
             return RTX_OK;
         default:
             return set_err(ctx, RTX_ERR_INVALID, "unknown option");
@@ -796,9 +785,8 @@ static int bind_scratch(rtx_ctx* ctx) {
     CU(cudaFuncSetAttribute(prefix_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->prefix_smem));
     CU(cudaFuncSetAttribute(lineage_walk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->walk_smem));
     CU(cudaFuncSetAttribute(lineage_walk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->walk_smem));
-    CU(cudaFuncSetAttribute(lineage_bfs_kernel<kBfsThreadsDefault, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->bfs_smem));
-    CU(cudaFuncSetAttribute(lineage_bfs_kernel<kBfsThreadsDefault, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->bfs_smem));
-    CU(cudaFuncSetAttribute(lineage_bfs_kernel<128, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->bfs_smem));
+    CU(cudaFuncSetAttribute(lineage_bfs_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->bfs_smem));
+    CU(cudaFuncSetAttribute(lineage_bfs_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->bfs_smem));
     ctx->cur_stream = ctx->stream;
     ctx->cur_counts = ctx->d_counts.as<u16>();
     ctx->cur_sc = &ctx->sc;
@@ -1002,126 +990,81 @@ RTX_API int rtx_batch_upload(rtx_ctx* ctx, const rtx_batch* batch) {
 // ---------------------------------------------------------------------------------------------------------
 // kernels
 // ---------------------------------------------------------------------------------------------------------
-// Launch geometry of the bit-row kernel.  `tune` (RTX_OPT_HITCOUNT_TUNE) = V + 10*PF + 100*nwarps, 0 = default.
-template <int V, int NP, bool PF>
-static cudaError_t launch_hitcount(rtx_ctx* c, int q_base, int qb, int nwarps_opt) {
-    const int n_tiles = (int)(c->ix.row_words / (32 * V));
-    // L2 blocking: CTAs are scheduled query-fastest, so all queries of one reference tile group run together; the
-    // group's slice of the bit matrix (n_rows x tiles x 128*V bytes) should stay resident in the 126 MB L2.
-    int max_tiles = c->hit_max_tiles;
-    if (max_tiles <= 0) {
-        const double slice_bytes_per_tile = (double)c->n_rows * 32.0 * V * 4.0;
-        max_tiles = (int)std::min(64.0, std::max(4.0, std::floor(64e6 / slice_bytes_per_tile)));
-    }
-    const int groups = (n_tiles + max_tiles - 1) / max_tiles;
-    const int tiles_per_cta = (n_tiles + groups - 1) / groups;
-    // warps per CTA: the count in [4, 8] that wastes the fewest warp slots in the last round
-    int nwarps = nwarps_opt;
-    if (nwarps <= 0) {
-        double best = -1.0;
-        for (int w = 8; w >= 4; --w) {
-            const int rounds = (tiles_per_cta + w - 1) / w;
-            const double eff = (double)tiles_per_cta / (rounds * w);
-            if (eff > best + 1e-9) {
-                best = eff;
-                nwarps = w;
-            }
-        }
-    }
-    nwarps = std::max(1, std::min(nwarps, kHitThreads / 32));
-    const bool hist_global = (size_t)(kRowListCap + c->bv.hstride) * 4 > 200 * 1024;  // tens of thousands of 8-mers per query
-    const size_t smem = (size_t)(kRowListCap + (hist_global ? 0 : c->bv.hstride)) * 4;
-    cudaError_t e = cudaFuncSetAttribute(hitcount_bitrows_kernel<V, NP, PF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    dim3 grid(qb, groups);
-    c->hit_kernel = "hitcount_bitrows_kernel<" + std::to_string(V) + ", " + std::to_string(NP) + ", " + (PF ? "true" : "false") + ">";
-    hitcount_bitrows_kernel<V, NP, PF><<<grid, nwarps * 32, smem, c->cur_stream>>>(c->ix, c->bv, c->cur_counts, q_base, tiles_per_cta, n_tiles,
-                                                                                 hist_global ? 1 : 0);
-    return cudaGetLastError();
-}
-
-template <int V, bool PF>
-static cudaError_t launch_hitcount_np(rtx_ctx* c, int q_base, int qb, u32 kmax, int nwarps) {
-    if (kmax < (1u << 8)) return launch_hitcount<V, 8, PF>(c, q_base, qb, nwarps);
-    if (kmax < (1u << 10)) return launch_hitcount<V, 10, PF>(c, q_base, qb, nwarps);
-    if (kmax < (1u << 11)) return launch_hitcount<V, 11, PF>(c, q_base, qb, nwarps);
-    if (kmax < (1u << 13)) return launch_hitcount<V, 13, PF>(c, q_base, qb, nwarps);
-    return launch_hitcount<V, 16, PF>(c, q_base, qb, nwarps);
-}
-
 // L2 blocking shared by both bit-row kernels: CTAs are scheduled query-fastest, so all queries of one reference tile group
-// run together; the group's slice of the bit matrix (n_rows x tiles x 128*V bytes) should stay resident in the 126 MB L2.
-static void hit_tile_groups(const rtx_ctx* c, int V, int* n_tiles, int* groups, int* tiles_per_cta) {
-    *n_tiles = (int)(c->ix.row_words / (32 * V));
+// run together; the group's slice of the bit matrix (n_rows x tiles x 256 bytes) should stay resident in the 126 MB L2.
+static void hit_tile_groups(const rtx_ctx* c, int* n_tiles, int* groups, int* tiles_per_cta) {
+    *n_tiles = (int)(c->ix.row_words / (32 * kLaneWords));
     int max_tiles = c->hit_max_tiles;
     if (max_tiles <= 0) {
-        const double slice_bytes_per_tile = (double)c->n_rows * 32.0 * V * 4.0;
+        const double slice_bytes_per_tile = (double)c->n_rows * 32.0 * kLaneWords * 4.0;
         max_tiles = (int)std::min(64.0, std::max(4.0, std::floor(64e6 / slice_bytes_per_tile)));
     }
     *groups = (*n_tiles + max_tiles - 1) / max_tiles;
     *tiles_per_cta = (*n_tiles + *groups - 1) / *groups;
 }
 
-// query-group kernel: G queries per CTA (one per warp) in lockstep over row-id chunks sized to the L1
+// single-query kernel: one query per CTA, its tile group's tiles spread over the warps
 template <int NP>
-static cudaError_t launch_hitcount_group(rtx_ctx* c, int q_base, int qb, int G) {
-    constexpr int V = 2;
+static cudaError_t launch_hitcount(rtx_ctx* c, int q_base, int qb) {
     int n_tiles, groups, tiles_per_cta;
-    hit_tile_groups(c, V, &n_tiles, &groups, &tiles_per_cta);
-    const u32 ks = c->bv.kstride, hs = c->bv.hstride;
-    // lockstep chunks: measured on C2 (profiles/r01_hitcount_group_sweep.txt) the barriers cost more than the L1 hits save
-    // (G16: L1 hit rate 48 %, L2 throughput 22 %, but 7.6 ms against 5.6 ms without barriers), so the default is none.
-    int n_chunks = c->hit_chunks > 0 ? c->hit_chunks : 1;
-    n_chunks = std::max(1, std::min(n_chunks, 4096));
-    const u32 chunk_rows = (c->n_rows + n_chunks - 1) / n_chunks + 1;
-    const size_t smem = (size_t)G * (ks + hs) * 4 + (size_t)G * n_chunks * 2 + 16;
-    dim3 grid((qb + G - 1) / G, groups);
-    auto go = [&](auto kernel) -> cudaError_t {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        const u32 n_seg = (u32)(c->ix.n_pad / kPrefixSeg);
-        u16* segmax = const_cast<u16*>(seg_max(*c->cur_sc, 0, n_seg));
-        kernel<<<grid, G * 32, smem, c->cur_stream>>>(c->ix, c->bv, c->cur_counts, q_base, qb, tiles_per_cta, n_tiles, chunk_rows, n_chunks, segmax,
-                                                    c->cur_sc->segoff_stride * 4);
-        c->segmax_valid = true;
-        return cudaGetLastError();
-    };
-    // hit_tune: 0 default, 1 = .v2 row loads that bypass the L1, 2 = .v2 row loads through the L1 (the round-1 kernel),
-    // 3 = one-line loads (lane words l and l + 32) through the L1, 4 = one-line loads that bypass the L1
-    const int mode = c->hit_tune ? c->hit_tune : 2;
-    const bool lockstep = n_chunks > 1, l1a = lockstep || mode == 2 || mode == 3, split = !lockstep && (mode == 3 || mode == 4);
-    c->hit_kernel = "hitcount_group_kernel<2, " + std::to_string(NP) + ", " + (lockstep ? "true" : "false") + ", " + std::to_string(kHitGroupMaxThreads) +
-                    ", 1, " + (l1a ? "true" : "false") + ", " + (split ? "true" : "false") + "> (" + std::to_string(G) + " queries per CTA)";
-    if (lockstep) return go(hitcount_group_kernel<V, NP, true, kHitGroupMaxThreads, 1>);
-    if (split) return l1a ? go(hitcount_group_kernel<V, NP, false, kHitGroupMaxThreads, 1, true, true>)
-                          : go(hitcount_group_kernel<V, NP, false, kHitGroupMaxThreads, 1, false, true>);
-    if (!l1a) return go(hitcount_group_kernel<V, NP, false, kHitGroupMaxThreads, 1, false>);  // L1 bypass (measured option)
-    return go(hitcount_group_kernel<V, NP, false, kHitGroupMaxThreads, 1>);
+    hit_tile_groups(c, &n_tiles, &groups, &tiles_per_cta);
+    // warps per CTA: the count in [4, 8] that wastes the fewest warp slots in the last round
+    int nwarps = 0;
+    double best = -1.0;
+    for (int w = 8; w >= 4; --w) {
+        const int rounds = (tiles_per_cta + w - 1) / w;
+        const double eff = (double)tiles_per_cta / (rounds * w);
+        if (eff > best + 1e-9) {
+            best = eff;
+            nwarps = w;
+        }
+    }
+    const bool hist_global = (size_t)(kRowListCap + c->bv.hstride) * 4 > 200 * 1024;  // tens of thousands of 8-mers per query
+    const size_t smem = (size_t)(kRowListCap + (hist_global ? 0 : c->bv.hstride)) * 4;
+    cudaError_t e = cudaFuncSetAttribute(hitcount_bitrows_kernel<NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    dim3 grid(qb, groups);
+    c->hit_kernel = "hitcount_bitrows_kernel<" + std::to_string(NP) + ">";
+    hitcount_bitrows_kernel<NP><<<grid, nwarps * 32, smem, c->cur_stream>>>(c->ix, c->bv, c->cur_counts, q_base, tiles_per_cta, n_tiles,
+                                                                          hist_global ? 1 : 0);
+    return cudaGetLastError();
 }
 
-static cudaError_t launch_hitcount_tuned(rtx_ctx* c, int q_base, int qb, u32 kmax) {
-    c->segmax_valid = false;  // only the query-group kernel leaves per-segment maxima
-    int G = c->hit_group;  // 0 = default
-    const bool force_group = G == 101;
-    if (force_group) G = 1;
+// query-group kernel: G queries per CTA (one per warp) over the same reference tiles
+template <int NP>
+static cudaError_t launch_hitcount_group(rtx_ctx* c, int q_base, int qb, int G) {
+    int n_tiles, groups, tiles_per_cta;
+    hit_tile_groups(c, &n_tiles, &groups, &tiles_per_cta);
+    const size_t smem = (size_t)G * (c->bv.kstride + c->bv.hstride) * 4;
+    cudaError_t e = cudaFuncSetAttribute(hitcount_group_kernel<NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    dim3 grid((qb + G - 1) / G, groups);
+    const u32 n_seg = (u32)(c->ix.n_pad / kPrefixSeg);
+    u16* segmax = const_cast<u16*>(seg_max(*c->cur_sc, 0, n_seg));
+    c->hit_kernel = "hitcount_group_kernel<" + std::to_string(NP) + "> (" + std::to_string(G) + " queries per CTA)";
+    hitcount_group_kernel<NP><<<grid, G * 32, smem, c->cur_stream>>>(c->ix, c->bv, c->cur_counts, q_base, qb, tiles_per_cta, n_tiles, segmax,
+                                                                   c->cur_sc->segoff_stride * 4);
+    c->segmax_valid = true;
+    return cudaGetLastError();
+}
+
+// kmax: the most 8-mers of a query in the sub-batch, which bounds the counts and so the bit planes (NP) the kernels keep
+static cudaError_t launch_hitcount_bitrows(rtx_ctx* c, int q_base, int qb, u32 kmax) {
     // queries per CTA: 4 on indexes of a few GB, 16 on large ones -- measured (profiles/r2_hitcount_group_by_index_size.txt): on 1 M x 650 bp
     // references (8.2 GB of bit rows) 16 queries per CTA are 5.8 % faster than 4 (more rows shared through the L1, less L2 traffic), on
     // 100 k references (0.8 GB) and on 500 k x 1500 bp (4.1 GB) they are 1-5 % slower
+    int G = c->hit_group;  // 0 = default
     if (G == 0) G = ((u64)c->n_rows * c->ix.row_words * 4 >= (6ull << 30)) ? 16 : 4;
     while (G > 1 && (size_t)G * (c->bv.kstride + c->bv.hstride) * 4 > 150 * 1024) G /= 2;  // long queries: smaller groups
-    if ((G > 1 || force_group) && qb >= G) {
-        if (kmax < (1u << 8)) return launch_hitcount_group<8>(c, q_base, qb, G);
-        if (kmax < (1u << 10)) return launch_hitcount_group<10>(c, q_base, qb, G);
-        if (kmax < (1u << 11)) return launch_hitcount_group<11>(c, q_base, qb, G);
-        if (kmax < (1u << 13)) return launch_hitcount_group<13>(c, q_base, qb, G);
-        return launch_hitcount_group<16>(c, q_base, qb, G);
+    const bool single = G == 1 || qb < G;
+    const int NP = kmax < (1u << 8) ? 8 : kmax < (1u << 10) ? 10 : kmax < (1u << 11) ? 11 : kmax < (1u << 13) ? 13 : 16;
+    switch (NP) {
+        case 8: return single ? launch_hitcount<8>(c, q_base, qb) : launch_hitcount_group<8>(c, q_base, qb, G);
+        case 10: return single ? launch_hitcount<10>(c, q_base, qb) : launch_hitcount_group<10>(c, q_base, qb, G);
+        case 11: return single ? launch_hitcount<11>(c, q_base, qb) : launch_hitcount_group<11>(c, q_base, qb, G);
+        case 13: return single ? launch_hitcount<13>(c, q_base, qb) : launch_hitcount_group<13>(c, q_base, qb, G);
+        default: return single ? launch_hitcount<16>(c, q_base, qb) : launch_hitcount_group<16>(c, q_base, qb, G);
     }
-    const int tune = c->hit_tune >= 10 ? c->hit_tune : 12;  // default: 2 words per lane, register double buffering
-    const int V = tune % 10 ? tune % 10 : 4;
-    const bool PF = (tune / 10) % 10 != 0;
-    const int nwarps = tune / 100;
-    if (V == 2) return PF ? launch_hitcount_np<2, true>(c, q_base, qb, kmax, nwarps) : launch_hitcount_np<2, false>(c, q_base, qb, kmax, nwarps);
-    return launch_hitcount_np<4, false>(c, q_base, qb, kmax, nwarps);
 }
 
 static int run_phase1(rtx_ctx* ctx, int q_base, int qb) {
@@ -1138,7 +1081,7 @@ static int run_phase1(rtx_ctx* ctx, int q_base, int qb) {
         hitcount_csr_kernel<<<grid, kCsrThreads, smem, ctx->cur_stream>>>(ctx->ix, ctx->bv, ctx->cur_counts, q_base);
         CU(cudaGetLastError());
     } else {
-        CU(launch_hitcount_tuned(ctx, q_base, qb, kmax));
+        CU(launch_hitcount_bitrows(ctx, q_base, qb, kmax));
     }
     return RTX_OK;
 }
@@ -1201,18 +1144,19 @@ static int begin_run(rtx_ctx* ctx) {
     return RTX_OK;
 }
 
-// tree walk of one shard's part of the tree: the level-synchronous kernel, then the depth-first walker for the queries it handed back
-// (RTX_OPT_WALK_VARIANT 1: depth-first walker only, as in round 1)
-static int launch_shard_walk(rtx_ctx* ctx, const ShardView& sv, const ProbScratch& sc, int q0, int qb, cudaStream_t st) {
+// tree walk of a sub-batch (SH: of this shard's part of the tree): the level-synchronous kernel, then the depth-first walker for the
+// queries it handed back (RTX_OPT_WALK_VARIANT 1: depth-first walker only)
+template <bool SH>
+static int launch_walk(rtx_ctx* ctx, const ShardView& sv, const ProbScratch& sc, int q0, int qb, cudaStream_t st) {
     LaunchTimer lt(ctx, RTX_K_WALK);
     const bool bfs = ctx->walk_variant != 1;
     if (bfs) {
         const u32 cap = ctx->walk_log_cap ? (u32)ctx->walk_log_cap : kBfsEntries;
-        lineage_bfs_kernel<kBfsThreadsDefault, true><<<qb, kBfsThreadsDefault, ctx->bfs_smem, st>>>(
-            ctx->ix, ctx->d_recs.as<NodeRec>(), ctx->bv, ctx->pool, sc, sv, q0, qb, cap, ctx->walk_variant == 3 ? 0 : ctx->walk_variant == 4 ? 2 : 1);
+        lineage_bfs_kernel<SH><<<qb, kBfsThreads, ctx->bfs_smem, st>>>(ctx->ix, ctx->d_recs.as<NodeRec>(), ctx->bv, ctx->pool, sc, sv, q0, qb, cap,
+                                                                     ctx->walk_variant == 3 ? 0 : ctx->walk_variant == 4 ? 2 : 1);
         CU(cudaGetLastError());
     }
-    lineage_walk_kernel<true><<<(qb + kWalkWarps - 1) / kWalkWarps, kWalkWarps * 32, ctx->walk_smem, st>>>(
+    lineage_walk_kernel<SH><<<(qb + kWalkWarps - 1) / kWalkWarps, kWalkWarps * 32, ctx->walk_smem, st>>>(
         ctx->ix, ctx->d_recs.as<NodeRec>(), ctx->bv, ctx->pool, sc, sv, q0, qb, bfs ? 1 : 0);
     CU(cudaGetLastError());
     return RTX_OK;
@@ -1269,21 +1213,8 @@ static int run_all(rtx_ctx* ctx) {
             if (rc2) return rc2;
         }
         {
-            LaunchTimer lt(ctx, RTX_K_WALK);
-            if (ctx->walk_variant != 1) {  // level-synchronous walk, then the depth-first walker for the queries it handed back
-                const u32 cap = ctx->walk_log_cap ? (u32)ctx->walk_log_cap : kBfsEntries;
-                if (ctx->walk_variant == 2)
-                    lineage_bfs_kernel<128, false><<<qb, 128, ctx->bfs_smem, ctx->cur_stream>>>(ctx->ix, ctx->d_recs.as<NodeRec>(), bv, ctx->pool,
-                                                                                                *ctx->cur_sc, ShardView{}, (int)q0, qb, cap, 1);
-                else
-                    lineage_bfs_kernel<kBfsThreadsDefault, false><<<qb, kBfsThreadsDefault, ctx->bfs_smem, ctx->cur_stream>>>(
-                        ctx->ix, ctx->d_recs.as<NodeRec>(), bv, ctx->pool, *ctx->cur_sc, ShardView{}, (int)q0, qb, cap,
-                        ctx->walk_variant == 3 ? 0 : ctx->walk_variant == 4 ? 2 : 1);
-                CU(cudaGetLastError());
-            }
-            lineage_walk_kernel<false><<<(qb + kWalkWarps - 1) / kWalkWarps, kWalkWarps * 32, ctx->walk_smem, ctx->cur_stream>>>(
-                ctx->ix, ctx->d_recs.as<NodeRec>(), bv, ctx->pool, *ctx->cur_sc, ShardView{}, (int)q0, qb, ctx->walk_variant != 1 ? 1 : 0);
-            CU(cudaGetLastError());
+            int rc2 = launch_walk<false>(ctx, ShardView{}, *ctx->cur_sc, (int)q0, qb, ctx->cur_stream);
+            if (rc2) return rc2;
         }
         if (ctx->tap_counts_host) {
             const u64 Ns = ctx->ix.shard_refs;
@@ -1563,7 +1494,7 @@ RTX_API int rtx_shard_phase3(rtx_ctx* ctx) {
         shard_combine_kernel<<<(nq + 127) / 128, 128, 0, ctx->stream>>>(ctx->sv, ctx->d_recs.as<NodeRec>(), (int)nq);
         CU(cudaGetLastError());
     }
-    rc = launch_shard_walk(ctx, ctx->sv, ctx->sc, 0, (int)nq, ctx->stream);
+    rc = launch_walk<true>(ctx, ctx->sv, ctx->sc, 0, (int)nq, ctx->stream);
     if (rc) return rc;
     ctx->cur_stream = ctx->stream;
     rc = order_results(ctx);
@@ -1800,7 +1731,7 @@ RTX_API int rtx_shard_run(rtx_ctx* ctx) {
                 CU(cudaGetLastError());
             }
         }
-        rc = launch_shard_walk(ctx, sv, *ctx->cur_sc, (int)q0, qb, st);
+        rc = launch_walk<true>(ctx, sv, *ctx->cur_sc, (int)q0, qb, st);
         if (rc) return rc;
         if (pipe) CU(cudaEventRecord(ctx->ev_post[slot], ctx->stream2));
     }

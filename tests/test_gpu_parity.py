@@ -296,6 +296,11 @@ def test_errors_are_loud(ctx):
     c2.close()
     with pytest.raises(capi.RtxError):
         ctx.upload_index_arrays(0, np.zeros(65537, np.uint64), np.zeros(1, np.uint32), [0], [0], [0], [0], [0], [1])
+    # options 5 and 8 are not assigned, walk variant 2 does not exist, a CTA holds at most 16 queries
+    for opt, value in [(5, 0), (8, 0), (capi.RTX_OPT_WALK_VARIANT, 2), (capi.RTX_OPT_HITCOUNT_GROUP, 101)]:
+        with pytest.raises(capi.RtxError) as ei:
+            ctx.set_option(opt, value)
+        assert ei.value.code == capi.RTX_ERR_INVALID
 
 
 # ---- full-size properties (BASELINE configs 2, 3, 4 at their full reference counts, reduced query counts) -----------------------
@@ -854,6 +859,7 @@ def test_documented_limits(oracle, ctx):
     _assert_integer_parity(o, dev, 3)
     _assert_result_parity(o, dev, ot, 3, max_tolerated_frac=1.0)
     assert dev.confidence.shape[1] == 32
+    assert ctx.hitcount_kernel_name().startswith("hitcount_bitrows_kernel<")  # fewer queries than a query group: the single-query kernel
     lin33, refs33 = db(33)
     with pytest.raises(capi.RtxError) as ei:
         ctx.upload_tree(capi.Tree.new(lin33, *_pack(oracle, refs33)))
@@ -888,6 +894,8 @@ def test_documented_limits(oracle, ctx):
         _assert_integer_parity(o, dev, 3)
         _assert_result_parity(o, dev, ot, 3, max_tolerated_frac=1.0)
         assert int(dev.n_kmers.max()) > length * 0.85
+        if length == 21000:  # row list and histogram too large for a warp's shared memory: the single-query kernel
+            assert ctx.hitcount_kernel_name().startswith("hitcount_bitrows_kernel<")
     # raxtax.rs:56 asserts at most 65 535 unique 8-mers; longer queries are refused, loudly
     with pytest.raises(capi.RtxError) as ei:
         ctx.classify(*_pack(oracle, [synth.BASE_CODES[rng.integers(0, 4, 70000)]]))

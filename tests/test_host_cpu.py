@@ -31,7 +31,7 @@ def test_device_abi_exports_every_declared_symbol():
     for n in names:
         assert hasattr(lib, n), n
     lib.rtx_abi_version.restype = C.c_int
-    assert lib.rtx_abi_version() == 3
+    assert lib.rtx_abi_version() == 4
 
 
 def test_host_abi_exports_every_declared_symbol():

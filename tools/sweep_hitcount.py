@@ -1,10 +1,9 @@
 """GPU micro-benchmark: hit-count kernel time on a workload for each geometry.
 
-usage: sweep_hitcount.py [workload] [configs]     configs = comma-separated words of letter+number fields, e.g.  G16C0,G8C12,G1T12M4
-   G = RTX_OPT_HITCOUNT_GROUP (queries per CTA; 1 = single-query kernel), C = RTX_OPT_HITCOUNT_CHUNKS, T = RTX_OPT_HITCOUNT_TUNE,
-   M = RTX_OPT_HITCOUNT_MAX_TILES, S = RTX_OPT_SUB_BATCH (queries per device sub-batch), W = RTX_OPT_WALK_VARIANT
-   P = RTX_OPT_PIPELINE (two-stream sub-batch pipeline)
-   (group kernel: T1 = row loads bypass the L1).  Every configuration's histograms are compared with the first one's (bit-exact).
+usage: sweep_hitcount.py [workload] [configs]     configs = comma-separated words of letter+number fields, e.g.  G16,G8S2048,G1M4
+   G = RTX_OPT_HITCOUNT_GROUP (queries per CTA; 1 = single-query kernel), M = RTX_OPT_HITCOUNT_MAX_TILES,
+   S = RTX_OPT_SUB_BATCH (queries per device sub-batch), W = RTX_OPT_WALK_VARIANT, P = RTX_OPT_PIPELINE (two-stream sub-batch pipeline)
+   Every configuration's histograms are compared with the first one's (bit-exact).
 """
 import json
 import os
@@ -26,8 +25,8 @@ ctx = capi.Context(0)
 ctx.upload_tree(tree)
 eo, eids = tree.exact_batch(ds.query_off, ds.query_codes)
 ctx.batch_upload(ds.query_off, ds.query_codes, eo, eids)
-OPT = {"G": capi.RTX_OPT_HITCOUNT_GROUP, "C": capi.RTX_OPT_HITCOUNT_CHUNKS, "T": capi.RTX_OPT_HITCOUNT_TUNE, "M": capi.RTX_OPT_HITCOUNT_MAX_TILES,
-       "S": capi.RTX_OPT_SUB_BATCH, "W": capi.RTX_OPT_WALK_VARIANT, "P": capi.RTX_OPT_PIPELINE}
+OPT = {"G": capi.RTX_OPT_HITCOUNT_GROUP, "M": capi.RTX_OPT_HITCOUNT_MAX_TILES, "S": capi.RTX_OPT_SUB_BATCH, "W": capi.RTX_OPT_WALK_VARIANT,
+       "P": capi.RTX_OPT_PIPELINE}
 ref = None
 ref_counts = None
 n_chk = min(192, ds.n_queries)
@@ -35,7 +34,7 @@ chk_off = ds.query_off[: n_chk + 1]
 chk_codes = ds.query_codes[: int(chk_off[-1])]
 chk_eo, chk_eids = tree.exact_batch(chk_off, chk_codes)
 for cfg in configs:
-    f = {k: int(v) for k, v in re.findall(r"([GCTMSWP])(\d+)", cfg)}
+    f = {k: int(v) for k, v in re.findall(r"([GMSWP])(\d+)", cfg)}
     for k, o in OPT.items():
         ctx.set_option(o, f.get(k, 0))
     ctx.batch_upload(ds.query_off, ds.query_codes, eo, eids)  # the sub-batch size is fixed at upload time
