@@ -42,6 +42,13 @@ typedef struct rtx_ctx rtx_ctx;
 /* flags of rtx_batch.flags -- the two switches that reach the hot path (raxtax.rs:17-18) */
 #define RTX_SKIP_EXACT_MATCHES 1u /* --skip-exact-matches: zero the counters of exact matches (raxtax.rs:65-68) */
 #define RTX_RAW_CONFIDENCE 2u     /* --raw-confidence: disable the one-exact-match override (raxtax.rs:73-84) */
+/* --strand both: every query is classified in the orientation that shares more 8-mers with some reference.  With M(x) = the largest
+ * hit count of sequence x (after the skip zeroing), query s is classified as its reverse complement rc(s) iff M(rc(s)) > M(s); every
+ * tie (K = 0 reads, palindromes) stays as given.  "Classified as x" is exactly the classification of query x, exact matches of x
+ * included, so exact_offsets then has 2 * n_queries + 1 entries: [0, n) the queries as given, [n, 2n) their reverse complements
+ * (entry n + q = the exact matches of rc(query q)).  Every output (result lines, global_signal, all taps) describes the classified
+ * orientation; rtx_batch_strands tells which one it was.  Not available in reference-sharded mode. */
+#define RTX_BOTH_STRANDS 4u
 
 /* hit-count kernel variants (rtx_ctx_set_option(RTX_OPT_HITCOUNT_VARIANT)) */
 #define RTX_HITCOUNT_BITROWS 0 /* bit-row positional popcount (default) */
@@ -136,7 +143,7 @@ const char* rtx_hitcount_kernel_name(const rtx_ctx* ctx);
 /* ---- query batch (src/raxtax.rs:14-22: `queries: &[(String, Vec<u8>)]` minus the labels) ----------------
  * seq_codes are the 4-bit one-hot codes of parser.rs:11-34.  exact_ids[exact_offsets[q]..exact_offsets[q+1])
  * is `tree.sequences.get(query_sequence)` (raxtax.rs:42) looked up by the host; exact_offsets may be NULL
- * when no query has an exact match.
+ * when no query has an exact match.  With RTX_BOTH_STRANDS in flags exact_offsets has 2 * n_queries + 1 entries.
  */
 typedef struct {
     uint32_t n_queries;
@@ -191,6 +198,9 @@ int rtx_batch_download(rtx_ctx* ctx, rtx_results* results);
  * (waits for A only) while B runs -- see rxh_raxtax in raxtax_host.cpp.  The reference's counterpart is rayon keeping every core
  * busy with the next chunk (raxtax.rs:35-39). */
 int rtx_batch_slot(rtx_ctx* ctx, int slot);
+/* Orientation each query of a RTX_BOTH_STRANDS batch was classified in: strand[q] = 0 as given, 1 reverse complement.  Valid after
+ * rtx_batch_download (or rtx_classify_batch) of such a batch in the active slot; RTX_ERR_INVALID otherwise. */
+int rtx_batch_strands(rtx_ctx* ctx, uint8_t* strand /* [n_queries] */);
 
 /* ---- reference-sharded mode (north_star: NCCL all-reduce of the per-query count histograms) -------------
  * Every rank uploads the same batch.  Per batch (which must fit one sub-batch):
@@ -246,6 +256,9 @@ typedef struct {
     double total_ms;     /* sum of CUDA-event durations (only with RTX_OPT_PROFILE) */
 } rtx_kernel_stat;
 
+/* RTX_K_HITCOUNT counts both passes of a RTX_BOTH_STRANDS batch; RTX_K_FIXUP the skip-exact fix-up of either strand and, with
+ * RTX_BOTH_STRANDS, the strand decision behind it (strand_select_kernel: M of both strands, the winners' rows copied over the query's;
+ * strand_exact_kernel: the exact-match lists of the classified orientations) */
 enum { RTX_K_KMERS = 0, RTX_K_HITCOUNT = 1, RTX_K_FIXUP = 2, RTX_K_PROB = 3, RTX_K_INDEX = 4, RTX_K_WALK = 5, RTX_K_PREFIX = 6,
        RTX_K_ALLREDUCE = 7 /* histogram all-reduce */, RTX_K_ALLGATHER = 8 /* straddler records, result offsets */,
        RTX_K_SHARD = 9 /* record / combine / merge kernels */, RTX_K_GATHER = 10 /* result lines -> root */, RTX_K_COUNT = 11 };

@@ -121,6 +121,15 @@ int rxh_raxtax_multi(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queries* quer
                      int raw_confidence, size_t chunk_size, rxh_sender sender, void* sender_user, int tsv, rxh_logger logger,
                      void* logger_user, int* warnings);
 
+/* rxh_raxtax_multi with every query classified in the orientation that shares more 8-mers with some reference (--strand both,
+ * RTX_BOTH_STRANDS in include/raxtax_b200.h): per distinct sequence the host also looks up the exact matches of its reverse complement;
+ * the exact-match log lines and the "differ above the leafs" warning are those of the classified orientation (written once the
+ * batch's strands are known); every line of the primary and the tsv string ends in a strand column (`\t+` as given, `\t-` reverse
+ * complement) and the tsv line carries the sequence in the classified orientation.  Not available over a reference-sharded index. */
+int rxh_raxtax_both_strands(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queries* queries, const rxh_tree* tree, int skip_exact_matches,
+                            int raw_confidence, size_t chunk_size, rxh_sender sender, void* sender_user, int tsv, rxh_logger logger,
+                            void* logger_user, int* warnings);
+
 /* raxtax::raxtax over a reference-sharded index (BASELINE config 5: databases too large to replicate) with all shards driven by this
  * process: ctxs[r] holds shard r of n_ctx (rxh_tree_upload_sharded).  When every shard sits on its own GPU the contexts are joined into
  * an NCCL communicator and one driver thread per rank calls rtx_shard_run / rtx_shard_gather (histogram all-reduce, record all-gather

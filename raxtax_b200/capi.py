@@ -19,7 +19,7 @@ from . import _build
 u8p, u16p, u32p, u64p, f64p = (C.POINTER(t) for t in (C.c_uint8, C.c_uint16, C.c_uint32, C.c_uint64, C.c_double))
 
 RTX_OK, RTX_ERR_INVALID, RTX_ERR_CUDA, RTX_ERR_NO_DEVICE, RTX_ERR_NO_INDEX, RTX_ERR_UNSUPPORTED, RTX_ERR_ASSERT = 0, -1, -2, -3, -4, -5, -6
-RTX_SKIP_EXACT_MATCHES, RTX_RAW_CONFIDENCE = 1, 2
+RTX_SKIP_EXACT_MATCHES, RTX_RAW_CONFIDENCE, RTX_BOTH_STRANDS = 1, 2, 4
 RTX_HITCOUNT_BITROWS, RTX_HITCOUNT_CSR = 0, 1
 RTX_OPT_HITCOUNT_VARIANT, RTX_OPT_SUB_BATCH, RTX_OPT_KEEP_CSR, RTX_OPT_PROFILE, RTX_OPT_HITCOUNT_MAX_TILES = 1, 2, 3, 4, 6
 RTX_OPT_HITCOUNT_GROUP, RTX_OPT_WALK_VARIANT, RTX_OPT_WALK_LOG_CAP, RTX_OPT_PIPELINE = 7, 9, 10, 11
@@ -30,6 +30,7 @@ DEVICE_SYMBOLS = [
     "rtx_abi_version", "rtx_ctx_create", "rtx_ctx_destroy", "rtx_last_error", "rtx_ctx_set_option", "rtx_ctx_stream", "rtx_ctx_device",
     "rtx_ctx_synchronize", "rtx_host_alloc", "rtx_host_free", "rtx_index_upload", "rtx_index_n_refs", "rtx_index_shard_refs", "rtx_index_max_levels", "rtx_batch_sub_batch",
     "rtx_index_device_bytes", "rtx_index_bitrow_bytes", "rtx_hitcount_kernel_name", "rtx_classify_batch", "rtx_batch_upload", "rtx_batch_run", "rtx_batch_download", "rtx_batch_slot",
+    "rtx_batch_strands",
     "rtx_shard_phase1", "rtx_shard_hist_buffer", "rtx_shard_phase2", "rtx_shard_records_buffers", "rtx_shard_phase3", "rtx_shard_exchange_hist_local", "rtx_shard_exchange_records_local",
     "rtx_comm_unique_id", "rtx_comm_init", "rtx_comm_destroy", "rtx_shard_run", "rtx_shard_gather", "rtx_shard_classify",
     "rtx_profile_reset", "rtx_profile_get",
@@ -38,7 +39,7 @@ DEVICE_SYMBOLS = [
 HOST_SYMBOLS = [
     "rxh_last_error", "rxh_tree_from_fasta", "rxh_tree_from_file", "rxh_queries_from_file", "rxh_tree_from_bin", "rxh_tree_save_bin", "rxh_queries_skip", "rxh_tree_new", "rxh_tree_free", "rxh_tree_num_tips", "rxh_tree_lineage",
     "rxh_tree_csr", "rxh_tree_build_kmer_map", "rxh_tree_has_kmer_map", "rxh_tree_exact", "rxh_tree_index_desc", "rxh_tree_upload", "rxh_tree_upload_sharded", "rxh_queries_from_fasta", "rxh_queries_new",
-    "rxh_queries_free", "rxh_queries_len", "rxh_queries_label", "rxh_queries_arrays", "rxh_raxtax", "rxh_raxtax_multi", "rxh_raxtax_sharded", "rxh_merge_shard_results", "rxh_exact_batch", "rxh_count_sender", "rxh_count_logger", "rxh_format_fixed", "rxh_release_buffers", "rxh_plan_chunks",
+    "rxh_queries_free", "rxh_queries_len", "rxh_queries_label", "rxh_queries_arrays", "rxh_raxtax", "rxh_raxtax_multi", "rxh_raxtax_both_strands", "rxh_raxtax_sharded", "rxh_merge_shard_results", "rxh_exact_batch", "rxh_count_sender", "rxh_count_logger", "rxh_format_fixed", "rxh_release_buffers", "rxh_plan_chunks",
 ]
 
 
@@ -120,6 +121,7 @@ def device_lib():
     L.rtx_batch_run.argtypes = [C.c_void_p]
     L.rtx_batch_slot.argtypes = [C.c_void_p, C.c_int]
     L.rtx_batch_download.argtypes = [C.c_void_p, C.POINTER(ResultsStruct)]
+    L.rtx_batch_strands.argtypes = [C.c_void_p, u8p]
     for f in ("rtx_shard_phase1", "rtx_shard_phase2", "rtx_shard_phase3", "rtx_profile_reset"):
         getattr(L, f).argtypes = [C.c_void_p]
     L.rtx_shard_hist_buffer.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]
@@ -192,6 +194,8 @@ def host_lib():
                              LOGGER, C.c_void_p, C.POINTER(C.c_int)]
     L.rxh_raxtax_multi.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, SENDER, C.c_void_p,
                                    C.c_int, LOGGER, C.c_void_p, C.POINTER(C.c_int)]
+    L.rxh_raxtax_both_strands.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, SENDER,
+                                          C.c_void_p, C.c_int, LOGGER, C.c_void_p, C.POINTER(C.c_int)]
     L.rxh_raxtax_sharded.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, SENDER, C.c_void_p,
                                      C.c_int, LOGGER, C.c_void_p, C.POINTER(C.c_int)]
     L.rxh_merge_shard_results.argtypes = [C.c_size_t, C.c_size_t, C.c_uint32, C.POINTER(u32p), C.POINTER(u32p), C.POINTER(u8p), C.POINTER(f64p),
@@ -234,6 +238,7 @@ class ClassifyOutput:
     hist: np.ndarray | None = None
     kmers: np.ndarray | None = None
     probs: np.ndarray | None = None  # [nq, kmax + 1] normalised P(m) by count (valid where the histogram is non-zero)
+    strand: np.ndarray | None = None  # both-strand batches: u8 [nq], 0 = classified as given, 1 = as its reverse complement
 
     def for_query(self, q):
         a, b = int(self.result_begin[q]), int(self.result_begin[q + 1])
@@ -459,12 +464,25 @@ class Context:
         out.confidence, out.local_signal = out.confidence[:n], out.local_signal[:n]
         return out
 
-    def classify(self, seq_off, codes, exact_off=None, exact_ids=None, skip_exact=False, raw_conf=False, taps=(), out=None, shard_root=None) -> ClassifyOutput:
+    @staticmethod
+    def _flags(skip_exact, raw_conf, both_strands):
+        return (RTX_SKIP_EXACT_MATCHES if skip_exact else 0) | (RTX_RAW_CONFIDENCE if raw_conf else 0) | (RTX_BOTH_STRANDS if both_strands else 0)
+
+    def batch_strands(self, nq) -> np.ndarray:
+        """rtx_batch_strands: per query of the downloaded both-strand batch, 0 = classified as given, 1 = as its reverse complement."""
+        s = np.zeros(max(nq, 1), np.uint8)
+        self._check(device_lib().rtx_batch_strands(self._h, _ptr(s, C.c_uint8)))
+        return s[:nq]
+
+    def classify(self, seq_off, codes, exact_off=None, exact_ids=None, skip_exact=False, raw_conf=False, taps=(), out=None, shard_root=None,
+                 both_strands=False) -> ClassifyOutput:
         """rtx_classify_batch: H2D + kernels + D2H in one call.  out = pinned_results(...) reuses page-locked result buffers.
         shard_root = r: rtx_shard_classify instead (reference-sharded mode over NCCL, every rank calls it with the same batch; the
-        final lines come back on rank r, nothing on the others)."""
+        final lines come back on rank r, nothing on the others).  both_strands: every query is classified in the orientation that
+        shares more 8-mers with some reference (RTX_BOTH_STRANDS); exact_off then has 2n + 1 entries (Tree.exact_batch_both_strands)
+        and the result's .strand tells the orientation."""
         L = device_lib()
-        flags = (RTX_SKIP_EXACT_MATCHES if skip_exact else 0) | (RTX_RAW_CONFIDENCE if raw_conf else 0)
+        flags = self._flags(skip_exact, raw_conf, both_strands)
         b, keep = self._make_batch(seq_off, codes, exact_off, exact_ids, flags)
         nq = b.n_queries
         so = keep[0]
@@ -488,23 +506,25 @@ class Context:
                 self._cap_hint = cap
                 continue
             self._check(rc)
+            if both_strands:
+                out.strand = self.batch_strands(nq)
             return self._trim(out, int(r.n_results))
 
-    def batch_upload(self, seq_off, codes, exact_off=None, exact_ids=None, skip_exact=False, raw_conf=False):
-        flags = (RTX_SKIP_EXACT_MATCHES if skip_exact else 0) | (RTX_RAW_CONFIDENCE if raw_conf else 0)
+    def batch_upload(self, seq_off, codes, exact_off=None, exact_ids=None, skip_exact=False, raw_conf=False, both_strands=False):
+        flags = self._flags(skip_exact, raw_conf, both_strands)
         b, keep = self._make_batch(seq_off, codes, exact_off, exact_ids, flags)
         self._check(device_lib().rtx_batch_upload(self._h, C.byref(b)))
         so = keep[0]
         if not hasattr(self, "_batch_infos"):
             self._batch_infos = {}
-        self._batch_infos[getattr(self, "_slot", 0)] = (b.n_queries, int((so[1:] - so[:-1]).max()) if b.n_queries else 0)
+        self._batch_infos[getattr(self, "_slot", 0)] = (b.n_queries, int((so[1:] - so[:-1]).max()) if b.n_queries else 0, both_strands)
 
     def batch_run(self):
         self._check(device_lib().rtx_batch_run(self._h))
 
     def batch_download(self, taps=()) -> ClassifyOutput:
         L = device_lib()
-        nq, max_len = self._batch_infos[getattr(self, "_slot", 0)]
+        nq, max_len, both_strands = self._batch_infos[getattr(self, "_slot", 0)]
         cap = max(nq * 8 + 64, getattr(self, "_cap_hint", 0))
         while True:
             out, r = self._alloc_results(nq, cap, max_len, taps)
@@ -514,6 +534,8 @@ class Context:
                 self._cap_hint = cap
                 continue
             self._check(rc)
+            if both_strands:
+                out.strand = self.batch_strands(nq)
             return self._trim(out, int(r.n_results))
 
     def profile_reset(self):
@@ -674,6 +696,18 @@ class Tree:
                 return eo, ids[:tot].copy()
             cap = int(tot)
 
+    def exact_batch_both_strands(self, seq_off, codes):
+        """exact_batch for a both-strand batch (RTX_BOTH_STRANDS): 2n + 1 offsets, [0, n) the queries as given, [n, 2n) their
+        reverse complements."""
+        from .synth import reverse_complement_batch
+
+        seq_off = np.asarray(seq_off, np.uint64)
+        codes = np.asarray(codes, np.uint8)
+        rc = reverse_complement_batch(seq_off - seq_off[0], codes[int(seq_off[0]): int(seq_off[-1])])
+        base = seq_off - seq_off[0]
+        both_off = np.concatenate([base, base[1:] + base[-1]])
+        return self.exact_batch(both_off, np.concatenate([codes[int(seq_off[0]): int(seq_off[-1])], rc]))
+
     def index_arrays(self) -> dict:
         self.build_kmer_map()
         d = IndexDesc()
@@ -741,9 +775,14 @@ class Queries:
         return o, c
 
 
-def raxtax(ctx: Context, queries: Queries, tree: Tree, skip_exact_matches=False, raw_confidence=False, chunk_size=0, tsv=False, sharded=False):
+def raxtax(ctx: Context, queries: Queries, tree: Tree, skip_exact_matches=False, raw_confidence=False, chunk_size=0, tsv=False, sharded=False,
+           both_strands=False):
     """raxtax::raxtax (raxtax.rs:14-97).  Returns (results, log_lines, warnings) where results is the list of
-    (query_label, primary_results, tsv_results_or_None) tuples the reference sends to its writer thread."""
+    (query_label, primary_results, tsv_results_or_None) tuples the reference sends to its writer thread.  both_strands: every query
+    is classified in the orientation that shares more 8-mers with some reference (rxh_raxtax_both_strands, one or several contexts);
+    every line then ends in a strand column (`+` / `-`)."""
+    if both_strands and sharded:
+        raise ValueError("both_strands is not available over a reference-sharded index")
     sent, logs = [], []
 
     def _send(_u, label, primary, tsv_s):
@@ -754,7 +793,12 @@ def raxtax(ctx: Context, queries: Queries, tree: Tree, skip_exact_matches=False,
         logs.append((level, msg.decode()))
 
     warn = C.c_int(0)
-    if sharded:  # ctx = the shards' contexts in shard order (upload_tree_sharded): rxh_raxtax_sharded, results in query order
+    if both_strands:
+        ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
+        arr = (C.c_void_p * len(ctxs))(*[c._h for c in ctxs])
+        rc = host_lib().rxh_raxtax_both_strands(arr, len(ctxs), queries._h, tree._h, int(skip_exact_matches), int(raw_confidence), int(chunk_size),
+                                                SENDER(_send), None, int(tsv), LOGGER(_log), None, C.byref(warn))
+    elif sharded:  # ctx = the shards' contexts in shard order (upload_tree_sharded): rxh_raxtax_sharded, results in query order
         arr = (C.c_void_p * len(ctx))(*[c._h for c in ctx])
         rc = host_lib().rxh_raxtax_sharded(arr, len(ctx), queries._h, tree._h, int(skip_exact_matches), int(raw_confidence), int(chunk_size),
                                            SENDER(_send), None, int(tsv), LOGGER(_log), None, C.byref(warn))

@@ -166,8 +166,53 @@ __global__ void __launch_bounds__(256) bitrows_from_seq_kernel(const u64* __rest
 // =========================================================================================================
 // K1: one CTA (128 threads) per query.  A 65 536-bit bitmap in shared memory is both the dedup set and the
 // sort: scanning it in word order emits the unique k-mers ascending (utils.rs:39).
+// kmers_both_kernel (--strand both, RTX_BOTH_STRANDS): the same pass also sets rc16(k) in a second bitmap and emits
+// the 8-mers of the reverse complement as virtual query n_queries + q.
 // =========================================================================================================
 constexpr int kKmerThreads = 128;
+
+// the 8-mer of the reverse complement strand at the same window: complement every base (A 0 <-> T 3, C 1 <-> G 2, i.e. x ^ 3)
+// and reverse the order of the eight 2-bit groups
+__host__ __device__ __forceinline__ u32 rc16(u32 k) {
+    u32 x = (k ^ 0xFFFFu) & 0xFFFFu;
+    x = ((x >> 2) & 0x3333u) | ((x & 0x3333u) << 2);
+    x = ((x >> 4) & 0x0F0Fu) | ((x & 0x0F0Fu) << 4);
+    return ((x >> 8) & 0x00FFu) | ((x & 0x00FFu) << 8);
+}
+
+// ordered compaction of one 65 536-bit k-mer set into query q's k-mer list, row list, K and padded row count;
+// thread t owns bitmap words [16t, 16t+16)
+__device__ __forceinline__ void kmers_compact(const IndexView& ix, const BatchView& b, const u32* bitmap, u32* wsum, int q, int tid) {
+    u32 cnt = 0, cnt_present = 0;
+#pragma unroll
+    for (int w = 0; w < 16; ++w) {
+        u32 x = bitmap[tid * 16 + w];
+        cnt += __popc(x);
+        cnt_present += __popc(x & ix.present[tid * 16 + w]);
+    }
+    u32 total, total_present;
+    u32 pos = block_scan_excl(cnt, wsum, tid, kKmerThreads / 32, &total);
+    u32 pos2 = block_scan_excl(cnt_present, wsum, tid, kKmerThreads / 32, &total_present);
+    u16* kout = b.kmers + (size_t)q * b.kstride;
+    u32* rout = b.rows + (size_t)q * b.kstride;
+    for (int w = 0; w < 16; ++w) {
+        u32 x = bitmap[tid * 16 + w];
+        while (x) {
+            u32 bit = __ffs(x) - 1;
+            x &= x - 1;
+            u32 kmer = (u32)(tid * 16 + w) * 32 + bit;
+            kout[pos++] = (u16)kmer;
+            u32 r = ix.rowmap[kmer];
+            if (r) rout[pos2++] = r;
+        }
+    }
+    u32 padded = (total_present + 15u) & ~15u;
+    if (tid < 16 && total_present + tid < padded) rout[total_present + tid] = 0;  // zero row
+    if (tid == 0) {
+        b.K[q] = (u16)total;
+        b.nrows[q] = padded;
+    }
+}
 
 __global__ void __launch_bounds__(kKmerThreads) kmers_kernel(IndexView ix, BatchView b) {
     __shared__ u32 bitmap[2048];
@@ -221,6 +266,39 @@ __global__ void __launch_bounds__(kKmerThreads) kmers_kernel(IndexView ix, Batch
         b.K[q] = (u16)total;
         b.nrows[q] = padded;
     }
+}
+
+// The window fold is written out again here rather than shared with kmers_kernel through a template or helper: the shared forms
+// compile kmers_kernel to different sm_100a code (16 more instructions: the compiler no longer keeps the warp index bound through
+// the helper), and the plus-mode kernel is meant to stay exactly as it is.  A change to the fold goes into both kernels.
+__global__ void __launch_bounds__(kKmerThreads) kmers_both_kernel(IndexView ix, BatchView b) {
+    __shared__ u32 bitmap[2 * 2048];  // [0, 2048) the query's 8-mers, [2048, 4096) those of its reverse complement
+    __shared__ u32 wsum[kKmerThreads / 32];
+    const int q = blockIdx.x, tid = threadIdx.x;
+    const u64 base = b.seq_off[q];
+    const u32 L = (u32)(b.seq_off[q + 1] - base);
+    for (int i = tid; i < 2 * 2048; i += kKmerThreads) bitmap[i] = 0;
+    __syncthreads();
+    if (L >= 8) {
+        for (u32 i = tid; i + 8 <= L; i += kKmerThreads) {  // sequence.windows(8)
+            u32 k = 0;
+            bool ok = true;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                u32 c = b.codes[base + i + j];
+                ok &= (c == 1u) | (c == 2u) | (c == 4u) | (c == 8u);
+                k |= ((u32)(__ffs(c) - 1) & 3u) << (14 - 2 * j);
+            }
+            if (ok) {
+                atomicOr(&bitmap[k >> 5], 1u << (k & 31));
+                const u32 r = rc16(k);
+                atomicOr(&bitmap[2048 + (r >> 5)], 1u << (r & 31));
+            }
+        }
+    }
+    __syncthreads();
+    kmers_compact(ix, b, bitmap, wsum, q, tid);
+    kmers_compact(ix, b, bitmap + 2048, wsum, (int)b.n_queries + q, tid);
 }
 
 // =========================================================================================================
@@ -659,6 +737,93 @@ __global__ void fixup_exact_kernel(IndexView ix, BatchView b, u16* __restrict__ 
             atomicSub(&hist[old], 1u);
             atomicAdd(&hist[0], 1u);
         }
+    }
+}
+
+// =========================================================================================================
+// K2'' (--strand both, RTX_BOTH_STRANDS): the orientation of every query of the sub-batch.  M(x), the largest hit count of
+// strand x after the skip zeroing, is the top non-empty bucket of x's histogram; the query is classified as its reverse
+// complement (virtual query n + q) iff M(rc) > M(fwd), every tie stays forward.  For a reverse winner this kernel leaves in
+// query q's place what K3-K5 and the taps read: the histogram row, the k-mer list, the count row and the per-segment maxima
+// (K is the same for both strands).  One CTA per query.
+// =========================================================================================================
+constexpr int kStrandThreads = 256;
+
+__global__ void __launch_bounds__(kStrandThreads, 1)
+    strand_select_kernel(IndexView ix, BatchView b, u16* __restrict__ counts, const u16* __restrict__ counts_rc, u16* __restrict__ segmax,
+                         size_t segmax_stride, const u16* __restrict__ segmax_rc, u32 n_seg, u8* __restrict__ strand, int q_base) {
+    __shared__ u32 smax[2];
+    const int tid = threadIdx.x, ql = blockIdx.x;
+    const int q = q_base + ql, qr = (int)b.n_queries + q;
+    const u32 K = b.K[q];
+    u32* __restrict__ hf = b.hist + (size_t)q * b.hstride;
+    const u32* __restrict__ hr = b.hist + (size_t)qr * b.hstride;
+    if (tid < 2) smax[tid] = 0;
+    __syncthreads();
+    u32 mf = 0, mr = 0;
+    for (u32 i = tid; i <= K; i += kStrandThreads) {  // ascending per thread: the last non-empty bucket seen is the thread's largest
+        if (hf[i]) mf = i;
+        if (hr[i]) mr = i;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        mf = max(mf, __shfl_xor_sync(kFullMask, mf, o));
+        mr = max(mr, __shfl_xor_sync(kFullMask, mr, o));
+    }
+    if ((tid & 31) == 0) {
+        atomicMax(&smax[0], mf);
+        atomicMax(&smax[1], mr);
+    }
+    __syncthreads();
+    const bool rc = smax[1] > smax[0];
+    if (tid == 0) strand[q] = rc ? 1 : 0;
+    if (!rc) return;
+    for (u32 i = tid; i <= K; i += kStrandThreads) hf[i] = hr[i];
+    u16* __restrict__ kf = b.kmers + (size_t)q * b.kstride;
+    const u16* __restrict__ kr = b.kmers + (size_t)qr * b.kstride;
+    for (u32 i = tid; i < K; i += kStrandThreads) kf[i] = kr[i];
+    // count rows: n_pad is a multiple of 4096 references, so whole 16-byte vectors
+    uint4* __restrict__ cf = reinterpret_cast<uint4*>(counts + (size_t)ql * ix.n_pad);
+    const uint4* __restrict__ cr = reinterpret_cast<const uint4*>(counts_rc + (size_t)ql * ix.n_pad);
+    for (u64 i = tid; i < ix.n_pad / 8; i += kStrandThreads) cf[i] = cr[i];
+    if (segmax_rc != nullptr)
+        for (u32 s = tid; s < n_seg; s += kStrandThreads) segmax[(size_t)ql * segmax_stride + s] = segmax_rc[(size_t)ql * n_seg + s];
+}
+
+// The exact matches of the classified orientation, as the override of the tree walk reads them (raxtax.rs:42,73-84):
+// sel_off[q + 1] = sel_off[q] + |exact matches of q's classified strand| over the sub-batch [q_base, q_base + q_count), ids behind.
+// The batch's exact_off / exact_ids hold the forward strands at [0, n) and the reverse complements at [n, 2n).  One CTA; the
+// sub-batches run in order on one stream, so sel_off[q_base] is already written (0 for the first).
+constexpr int kStrandScanThreads = 1024;
+
+__global__ void __launch_bounds__(kStrandScanThreads)
+    strand_exact_kernel(BatchView b, const u8* __restrict__ strand, u32* __restrict__ sel_off, u32* __restrict__ sel_ids, int q_base, int q_count) {
+    __shared__ u32 wsum[kStrandScanThreads / 32];
+    __shared__ u32 carry;
+    const int tid = threadIdx.x;
+    if (tid == 0) {
+        if (q_base == 0) sel_off[0] = 0;
+        carry = q_base == 0 ? 0u : sel_off[q_base];
+    }
+    __syncthreads();
+    for (int c0 = 0; c0 < q_count; c0 += kStrandScanThreads) {
+        const int ql = c0 + tid;
+        u32 src = 0, len = 0;
+        if (ql < q_count) {
+            const int q = q_base + ql;
+            const u32 s = strand[q] ? b.n_queries + (u32)q : (u32)q;
+            src = b.exact_off[s];
+            len = b.exact_off[s + 1] - src;
+        }
+        u32 total;
+        const u32 pos = carry + block_scan_excl(len, wsum, tid, kStrandScanThreads / 32, &total);
+        if (ql < q_count) {
+            sel_off[q_base + ql + 1] = pos + len;
+            for (u32 e = 0; e < len; ++e) sel_ids[pos + e] = b.exact_ids[src + e];
+        }
+        __syncthreads();
+        if (tid == 0) carry += total;
+        __syncthreads();
     }
 }
 

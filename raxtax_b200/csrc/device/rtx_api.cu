@@ -59,6 +59,11 @@ struct BatchState {
     u64 runs_since_download = 0;
     cudaEvent_t ev_up = nullptr, ev_done = nullptr;  // inputs are on the device / all kernels of the last run have finished
     bool up_pending = false;                          // ev_up was recorded and no run has waited for it yet
+    // --strand both (RTX_BOTH_STRANDS): the orientation of every query (K2''), the exact matches of the classified orientations
+    // (what the walk's override reads), the orientations as the last download brought them to the host
+    DevBuf d_strand, d_sel_off, d_sel_ids;
+    std::vector<u8> h_strand;
+    bool strands_ready = false;
     // reference-sharded mode over NCCL
     bool sub_batch_agreed = false;  // the ranks settled on one sub-batch size for this batch
     bool merged = false;            // rtx_shard_gather ran: d_ord_* hold the merged lines (root) / nothing (other ranks)
@@ -75,6 +80,11 @@ struct rtx_ctx : BatchState {
     cudaStream_t cur_stream = nullptr;  // what the launch helpers use: stream / slot of the sub-batch being issued
     u16* cur_counts = nullptr;
     bool segmax_valid = false;  // the last hit-count launch left per-segment maxima in cur_sc's aux area
+    u16* rc_segmax = nullptr;   // set: the query-group kernel writes them here instead (reverse strands, n_seg per query)
+    // RTX_BOTH_STRANDS without per-segment maxima (K4 then reads every count): the measured alternative to the reverse pass's own
+    // maxima area, selected by RTX_STRAND_SEGMAX=0 in the environment when the context is created (DESIGN.md §4, "Both strands")
+    bool strand_segmax = true;
+    bool no_segmax = false;     // set: the query-group kernel writes no per-segment maxima
     ProbScratch* cur_sc = nullptr;
     std::string err;
     std::string hit_kernel;  // the hit-count kernel instantiation of the last launch (rtx_hitcount_kernel_name)
@@ -278,6 +288,7 @@ RTX_API int rtx_ctx_create(int device_ordinal, rtx_ctx** out) {
         return set_err(nullptr, RTX_ERR_CUDA, m);
     }
     c->cur_stream = c->stream;
+    if (const char* e = getenv("RTX_STRAND_SEGMAX")) c->strand_segmax = strcmp(e, "0") != 0;
     // ln n! table: exact factorials up to 170, lgamma beyond (the reference's statrs::ln_factorial does the same)
     const u32 len = 98304 + 8;  // K + t <= 65535 + 32767
     std::vector<double> lf(len);
@@ -329,7 +340,8 @@ RTX_API void rtx_ctx_destroy(rtx_ctx* c) {
         DevBuf* sb[] = {&s.d_seq_off, &s.d_codes, &s.d_exact_off, &s.d_exact_ids, &s.d_K, &s.d_kmers, &s.d_rows, &s.d_nrows, &s.d_hist,
                         &s.d_pool_first, &s.d_pool_nlev, &s.d_pool_conf, &s.d_pool_local, &s.d_pool_used, &s.d_res_off, &s.d_res_cnt,
                         &s.d_global, &s.d_status, &s.d_hits, &s.d_ord_begin, &s.d_ord_first, &s.d_ord_nlev, &s.d_ord_conf, &s.d_ord_local,
-                        &s.d_counts, &s.d_counts1, &s.d_prob_big, &s.d_cbuf, &s.d_preb, &s.d_ptab, &s.d_segoff, &s.d_preb1, &s.d_ptab1, &s.d_segoff1};
+                        &s.d_counts, &s.d_counts1, &s.d_prob_big, &s.d_cbuf, &s.d_preb, &s.d_ptab, &s.d_segoff, &s.d_preb1, &s.d_ptab1, &s.d_segoff1,
+                        &s.d_strand, &s.d_sel_off, &s.d_sel_ids};
         for (DevBuf* b : sb) b->release();
         if (s.ev_up) cudaEventDestroy(s.ev_up);
         if (s.ev_done) cudaEventDestroy(s.ev_done);
@@ -802,6 +814,7 @@ RTX_API int rtx_batch_upload(rtx_ctx* ctx, const rtx_batch* batch) {
     CU(cudaSetDevice(ctx->device));
     ctx->has_batch = false;
     ctx->ran = false;
+    ctx->strands_ready = false;
     BatchView& bv = ctx->bv;
     bv = BatchView{};
     bv.n_queries = nq;
@@ -839,11 +852,13 @@ RTX_API int rtx_batch_upload(rtx_ctx* ctx, const rtx_batch* batch) {
     ctx->sc.lf_smem = lf_smem;
     ctx->max_len = max_len;
     ctx->total_codes = total;
+    const bool both = (batch->flags & RTX_BOTH_STRANDS) != 0;
+    const u32 nv = both ? 2 * nq : nq;  // virtual queries: with RTX_BOTH_STRANDS, n + q is the reverse complement of query q
     u64 total_exact = 0;
     if (batch->exact_offsets) {
-        for (u32 q = 0; q < nq; ++q) REQUIRE(batch->exact_offsets[q] <= batch->exact_offsets[q + 1], "exact_offsets must be non-decreasing");
+        for (u32 q = 0; q < nv; ++q) REQUIRE(batch->exact_offsets[q] <= batch->exact_offsets[q + 1], "exact_offsets must be non-decreasing");
         REQUIRE(batch->exact_offsets[0] == 0, "exact_offsets[0] must be 0");
-        total_exact = batch->exact_offsets[nq];
+        total_exact = batch->exact_offsets[nv];
         REQUIRE(total_exact == 0 || batch->exact_ids, "exact_ids is NULL");
         for (u64 e = 0; e < total_exact; ++e) REQUIRE(batch->exact_ids[e] < ctx->ix.n_refs, "exact id out of range");
     }
@@ -865,11 +880,11 @@ RTX_API int rtx_batch_upload(rtx_ctx* ctx, const rtx_batch* batch) {
     if (total) CU(cudaMemcpyAsync(ctx->d_codes.p, batch->seq_codes + batch->seq_offsets[0], total, cudaMemcpyHostToDevice, cs));
     ctx->prof.h2d_bytes += (nq + 1) * 8 + total;
     if (batch->exact_offsets) {
-        CU(ctx->d_exact_off.ensure((nq + 1) * 4));
+        CU(ctx->d_exact_off.ensure(((size_t)nv + 1) * 4));
         CU(ctx->d_exact_ids.ensure(std::max<u64>(total_exact, 1) * 4));
-        CU(cudaMemcpyAsync(ctx->d_exact_off.p, batch->exact_offsets, (nq + 1) * 4, cudaMemcpyHostToDevice, cs));
+        CU(cudaMemcpyAsync(ctx->d_exact_off.p, batch->exact_offsets, ((size_t)nv + 1) * 4, cudaMemcpyHostToDevice, cs));
         if (total_exact) CU(cudaMemcpyAsync(ctx->d_exact_ids.p, batch->exact_ids, total_exact * 4, cudaMemcpyHostToDevice, cs));
-        ctx->prof.h2d_bytes += (nq + 1) * 4 + total_exact * 4;
+        ctx->prof.h2d_bytes += ((u64)nv + 1) * 4 + total_exact * 4;
         bv.exact_off = ctx->d_exact_off.as<u32>();
         bv.exact_ids = ctx->d_exact_ids.as<u32>();
     }
@@ -880,12 +895,19 @@ RTX_API int rtx_batch_upload(rtx_ctx* ctx, const rtx_batch* batch) {
     bv.kstride = kstride;
     bv.hstride = hstride;
 
-    // per-query device arrays
-    CU(ctx->d_K.ensure(nq * 2));
-    CU(ctx->d_kmers.ensure((size_t)nq * kstride * 2));
-    CU(ctx->d_rows.ensure((size_t)nq * kstride * 4));
-    CU(ctx->d_nrows.ensure(nq * 4));
-    CU(ctx->d_hist.ensure((size_t)nq * hstride * 4));
+    // per-query device arrays (per virtual query: both strands with RTX_BOTH_STRANDS)
+    CU(ctx->d_K.ensure((size_t)nv * 2));
+    CU(ctx->d_kmers.ensure((size_t)nv * kstride * 2));
+    CU(ctx->d_rows.ensure((size_t)nv * kstride * 4));
+    CU(ctx->d_nrows.ensure((size_t)nv * 4));
+    CU(ctx->d_hist.ensure((size_t)nv * hstride * 4));
+    if (both) {
+        CU(ctx->d_strand.ensure(nq));
+        if (batch->exact_offsets) {
+            CU(ctx->d_sel_off.ensure(((size_t)nq + 1) * 4));
+            CU(ctx->d_sel_ids.ensure(std::max<u64>(total_exact, 1) * 4));
+        }
+    }
     bv.K = ctx->d_K.as<u16>();
     bv.kmers = ctx->d_kmers.as<u16>();
     bv.rows = ctx->d_rows.as<u32>();
@@ -911,13 +933,15 @@ RTX_API int rtx_batch_upload(rtx_ctx* ctx, const rtx_batch* batch) {
     // quarter of the memory that is free now, at most 48 GB and at least 2 GiB -- large sub-batches amortise the launch tails of
     // the walk and probability kernels (C3: 1 069 queries per sub-batch at the old fixed 2 GiB, ~6 000 now)
     const u64 per_query = ctx->ix.n_pad * 2;
+    // RTX_BOTH_STRANDS: a second count vector per query (the reverse complement) and its per-segment maxima
+    const u64 per_query_rc = both ? per_query + ctx->ix.n_pad / kPrefixSeg * 2 : 0;
     u64 sb = (u64)ctx->sub_batch_opt;
     if (!sb) {
         const u64 mem_free = ctx->mem_free_after_index;  // sampled once per index upload (cudaMemGetInfo costs ~1 ms per call)
         u64 budget = std::min<u64>(std::max<u64>(mem_free / 4, 2ull << 30), 48ull << 30);
         if (ctx->comm != nullptr && ctx->sv.n_shards > 1) budget = std::min<u64>(budget, std::max<u64>(mem_free / 5, 1ull << 30));  // two scratch slots
         const u64 scratch_per_query = per_query + ((u64)ctx->ix.n_pad / kBlkRefs + ctx->ix.n_pad / kPrefixSeg + ctx->ix.n_pad / kPrefixSeg / 64 + ctx->ix.n_pad / kPrefixSeg / 4 + 8 + hstride) * 8;
-        sb = std::max<u64>(1, budget / scratch_per_query);
+        sb = std::max<u64>(1, budget / (scratch_per_query + per_query_rc));
     }
     const bool may_pipe = ctx->pipeline_opt && ctx->sv.n_shards <= 1;
     if (!ctx->sub_batch_opt && may_pipe && nq >= 4096) sb = std::min<u64>(sb, std::max<u64>(1024, (nq + 3) / 4));  // >= 4 pipeline stages
@@ -926,7 +950,7 @@ RTX_API int rtx_batch_upload(rtx_ctx* ctx, const rtx_batch* batch) {
     ctx->two_slots = (may_pipe && nq > sb) || (ctx->comm != nullptr && ctx->sv.n_shards > 1 && nq > 1);
     ctx->sub_batch_agreed = false;
     ctx->merged = false;
-    ctx->need_counts = sb * per_query;
+    ctx->need_counts = sb * (per_query + per_query_rc);
 
     // probability kernel scratch
     ctx->prob_smem = smem;
@@ -1040,11 +1064,12 @@ static cudaError_t launch_hitcount_group(rtx_ctx* c, int q_base, int qb, int G) 
     if (e != cudaSuccess) return e;
     dim3 grid((qb + G - 1) / G, groups);
     const u32 n_seg = (u32)(c->ix.n_pad / kPrefixSeg);
-    u16* segmax = const_cast<u16*>(seg_max(*c->cur_sc, 0, n_seg));
+    u16* segmax = c->no_segmax ? nullptr : c->rc_segmax ? c->rc_segmax : const_cast<u16*>(seg_max(*c->cur_sc, 0, n_seg));
+    const size_t segmax_stride = c->rc_segmax ? (size_t)n_seg : c->cur_sc->segoff_stride * 4;
     c->hit_kernel = "hitcount_group_kernel<" + std::to_string(NP) + "> (" + std::to_string(G) + " queries per CTA)";
     hitcount_group_kernel<NP><<<grid, G * 32, smem, c->cur_stream>>>(c->ix, c->bv, c->cur_counts, q_base, qb, tiles_per_cta, n_tiles, segmax,
-                                                                   c->cur_sc->segoff_stride * 4);
-    c->segmax_valid = true;
+                                                                   segmax_stride);
+    c->segmax_valid = segmax != nullptr;
     return cudaGetLastError();
 }
 
@@ -1087,24 +1112,24 @@ static int run_phase1(rtx_ctx* ctx, int q_base, int qb) {
 }
 
 // K3 (P(m) tables) + K4 (prefix sums at node boundaries) of one sub-batch
-static int launch_prob(rtx_ctx* ctx, int q0, int qb) {
+static int launch_prob(rtx_ctx* ctx, const BatchView& bv, int q0, int qb) {
     {
         CU(cudaMemsetAsync(ctx->d_hits.as<unsigned long long>() + 1, 0, 8, ctx->cur_stream));  // the kernel's work counter
         LaunchTimer lt(ctx, RTX_K_PROB);
         const int grid = std::min(ctx->prob_slots, qb);
         if (ctx->cur_sc->big)
-            prob_table_kernel<true><<<grid, kProbThreads, 0, ctx->cur_stream>>>(ctx->ix, ctx->bv, ctx->pool, *ctx->cur_sc, q0, qb,
+            prob_table_kernel<true><<<grid, kProbThreads, 0, ctx->cur_stream>>>(ctx->ix, bv, ctx->pool, *ctx->cur_sc, q0, qb,
                                                                                 ctx->d_hits.as<unsigned long long>(),
                                                                                 ctx->d_hits.as<unsigned long long>() + 1);
         else
-            prob_table_kernel<false><<<grid, kProbThreads, ctx->prob_smem, ctx->cur_stream>>>(ctx->ix, ctx->bv, ctx->pool, *ctx->cur_sc, q0, qb,
+            prob_table_kernel<false><<<grid, kProbThreads, ctx->prob_smem, ctx->cur_stream>>>(ctx->ix, bv, ctx->pool, *ctx->cur_sc, q0, qb,
                                                                                             ctx->d_hits.as<unsigned long long>(),
                                                                                             ctx->d_hits.as<unsigned long long>() + 1);
         CU(cudaGetLastError());
     }
     {
         LaunchTimer lt(ctx, RTX_K_PREFIX);
-        prefix_kernel<<<qb, kPrefixThreads, ctx->prefix_smem, ctx->cur_stream>>>(ctx->ix, ctx->bv, *ctx->cur_sc, ctx->cur_counts, q0, qb,
+        prefix_kernel<<<qb, kPrefixThreads, ctx->prefix_smem, ctx->cur_stream>>>(ctx->ix, bv, *ctx->cur_sc, ctx->cur_counts, q0, qb,
                                                                                  ctx->segmax_valid ? 1 : 0);
         CU(cudaGetLastError());
     }
@@ -1147,18 +1172,55 @@ static int begin_run(rtx_ctx* ctx) {
 // tree walk of a sub-batch (SH: of this shard's part of the tree): the level-synchronous kernel, then the depth-first walker for the
 // queries it handed back (RTX_OPT_WALK_VARIANT 1: depth-first walker only)
 template <bool SH>
-static int launch_walk(rtx_ctx* ctx, const ShardView& sv, const ProbScratch& sc, int q0, int qb, cudaStream_t st) {
+static int launch_walk(rtx_ctx* ctx, const BatchView& bv, const ShardView& sv, const ProbScratch& sc, int q0, int qb, cudaStream_t st) {
     LaunchTimer lt(ctx, RTX_K_WALK);
     const bool bfs = ctx->walk_variant != 1;
     if (bfs) {
         const u32 cap = ctx->walk_log_cap ? (u32)ctx->walk_log_cap : kBfsEntries;
-        lineage_bfs_kernel<SH><<<qb, kBfsThreads, ctx->bfs_smem, st>>>(ctx->ix, ctx->d_recs.as<NodeRec>(), ctx->bv, ctx->pool, sc, sv, q0, qb, cap,
+        lineage_bfs_kernel<SH><<<qb, kBfsThreads, ctx->bfs_smem, st>>>(ctx->ix, ctx->d_recs.as<NodeRec>(), bv, ctx->pool, sc, sv, q0, qb, cap,
                                                                      ctx->walk_variant == 3 ? 0 : ctx->walk_variant == 4 ? 2 : 1);
         CU(cudaGetLastError());
     }
     lineage_walk_kernel<SH><<<(qb + kWalkWarps - 1) / kWalkWarps, kWalkWarps * 32, ctx->walk_smem, st>>>(
-        ctx->ix, ctx->d_recs.as<NodeRec>(), ctx->bv, ctx->pool, sc, sv, q0, qb, bfs ? 1 : 0);
+        ctx->ix, ctx->d_recs.as<NodeRec>(), bv, ctx->pool, sc, sv, q0, qb, bfs ? 1 : 0);
     CU(cudaGetLastError());
+    return RTX_OK;
+}
+
+// --strand both, after the forward hit counting of a sub-batch: hit counting of the reverse complements (virtual queries n + q) into
+// the second half of the slot's count buffer, then the strand decision (strand_select_kernel), which leaves in query q's place what
+// K3-K5 and the taps read of the orientation it is classified in, and the exact matches of those orientations for the walk's override
+static int run_reverse_strands(rtx_ctx* ctx, int q0, int qb) {
+    const BatchView& bv = ctx->bv;
+    const u32 nq = bv.n_queries;
+    const u32 n_seg = (u32)(ctx->ix.n_pad / kPrefixSeg);
+    u16* fwd = ctx->cur_counts;
+    u16* rev = fwd + (size_t)ctx->sub_batch * ctx->ix.n_pad;
+    u16* rev_segmax = rev + (size_t)ctx->sub_batch * ctx->ix.n_pad;
+    ctx->cur_counts = rev;
+    ctx->rc_segmax = rev_segmax;
+    const int rc = run_phase1(ctx, (int)(nq + q0), qb);
+    ctx->rc_segmax = nullptr;
+    ctx->cur_counts = fwd;
+    if (rc) return rc;
+    if ((bv.flags & RTX_SKIP_EXACT_MATCHES) && bv.exact_off) {
+        LaunchTimer lt(ctx, RTX_K_FIXUP);
+        fixup_exact_kernel<<<(qb + 127) / 128, 128, 0, ctx->cur_stream>>>(ctx->ix, bv, rev, (int)(nq + q0), qb);
+        CU(cudaGetLastError());
+    }
+    {
+        LaunchTimer lt(ctx, RTX_K_FIXUP);
+        // both passes ran the same hit-count kernel, so the forward maxima are there exactly when the reverse ones are
+        strand_select_kernel<<<qb, kStrandThreads, 0, ctx->cur_stream>>>(
+            ctx->ix, bv, fwd, rev, const_cast<u16*>(seg_max(*ctx->cur_sc, 0, n_seg)), ctx->cur_sc->segoff_stride * 4,
+            ctx->segmax_valid ? rev_segmax : nullptr, n_seg, ctx->d_strand.as<u8>(), q0);
+        CU(cudaGetLastError());
+        if (bv.exact_off) {
+            strand_exact_kernel<<<1, kStrandScanThreads, 0, ctx->cur_stream>>>(bv, ctx->d_strand.as<u8>(), ctx->d_sel_off.as<u32>(),
+                                                                             ctx->d_sel_ids.as<u32>(), q0, qb);
+            CU(cudaGetLastError());
+        }
+    }
     return RTX_OK;
 }
 
@@ -1172,12 +1234,21 @@ static int run_all(rtx_ctx* ctx) {
         int rc = begin_run(ctx);
         if (rc) return rc;
     }
-    CU(cudaMemsetAsync(ctx->d_hist.p, 0, (size_t)nq * bv.hstride * 4, ctx->stream));
+    const bool both = (bv.flags & RTX_BOTH_STRANDS) != 0;
+    ctx->no_segmax = both && !ctx->strand_segmax;
+    // what K3-K5 read: with both strands, the exact matches of the classified orientations (strand_exact_kernel)
+    BatchView tail = bv;
+    if (both && bv.exact_off) {
+        tail.exact_off = ctx->d_sel_off.as<u32>();
+        tail.exact_ids = ctx->d_sel_ids.as<u32>();
+    }
+    CU(cudaMemsetAsync(ctx->d_hist.p, 0, (size_t)(both ? 2 : 1) * nq * bv.hstride * 4, ctx->stream));
     CU(cudaMemsetAsync(ctx->d_pool_used.p, 0, 8, ctx->stream));
     CU(cudaMemsetAsync(ctx->d_hits.p, 0, 8, ctx->stream));
     {
         LaunchTimer lt(ctx, RTX_K_KMERS);
-        kmers_kernel<<<nq, kKmerThreads, 0, ctx->stream>>>(ctx->ix, bv);
+        if (both) kmers_both_kernel<<<nq, kKmerThreads, 0, ctx->stream>>>(ctx->ix, bv);
+        else kmers_kernel<<<nq, kKmerThreads, 0, ctx->stream>>>(ctx->ix, bv);
         CU(cudaGetLastError());
     }
     // Sub-batch pipeline: hit counting of sub-batch i runs on `stream`, everything behind it (probabilities, prefix sums,
@@ -1199,6 +1270,10 @@ static int run_all(rtx_ctx* ctx) {
             fixup_exact_kernel<<<(qb + 127) / 128, 128, 0, ctx->cur_stream>>>(ctx->ix, bv, ctx->cur_counts, (int)q0, qb);
             CU(cudaGetLastError());
         }
+        if (both) {
+            int rc2 = run_reverse_strands(ctx, (int)q0, qb);
+            if (rc2) return rc2;
+        }
         if (q0 + ctx->sub_batch >= nq) {  // the run's last hit-count launch: the batch in the other slot may start counting behind it
             CU(cudaEventRecord(ctx->ev_k2, ctx->stream));
             ctx->k2_recorded = true;
@@ -1209,11 +1284,11 @@ static int run_all(rtx_ctx* ctx) {
             CU(cudaStreamWaitEvent(ctx->stream2, ctx->ev_hit[slot], 0));
         }
         {
-            int rc2 = launch_prob(ctx, (int)q0, qb);
+            int rc2 = launch_prob(ctx, tail, (int)q0, qb);
             if (rc2) return rc2;
         }
         {
-            int rc2 = launch_walk<false>(ctx, ShardView{}, *ctx->cur_sc, (int)q0, qb, ctx->cur_stream);
+            int rc2 = launch_walk<false>(ctx, tail, ShardView{}, *ctx->cur_sc, (int)q0, qb, ctx->cur_stream);
             if (rc2) return rc2;
         }
         if (ctx->tap_counts_host) {
@@ -1275,7 +1350,8 @@ RTX_API int rtx_batch_download(rtx_ctx* ctx, rtx_results* res) {
     cudaStream_t cs = ctx->stream_cp;
     CU(cudaStreamWaitEvent(cs, ctx->ev_done, 0));  // this slot's kernels; the other slot may be running on `stream` meanwhile
     // round 1: per-query metadata through the pinned arena, one synchronisation
-    const size_t meta_bytes = 2 * 64 + ((size_t)nq + 1) * 4 + (size_t)nq * (4 + 4 + 2 + 8) + 6 * 64;
+    const bool both = (bv.flags & RTX_BOTH_STRANDS) != 0;
+    const size_t meta_bytes = 2 * 64 + ((size_t)nq + 1) * 4 + (size_t)nq * (4 + 4 + 2 + 8) + 6 * 64 + (both ? (size_t)nq + 64 : 0);
     CU(arena_reserve(ctx, meta_bytes));
     unsigned long long* h_used = (unsigned long long*)arena_take(ctx, 16);
     u32* h_begin = (u32*)arena_take(ctx, ((size_t)nq + 1) * 4);
@@ -1288,6 +1364,11 @@ RTX_API int rtx_batch_download(rtx_ctx* ctx, rtx_results* res) {
     CU(cudaMemcpyAsync(h_nrows, ctx->d_nrows.p, (size_t)nq * 4, cudaMemcpyDeviceToHost, cs));
     CU(d2h(ctx, res->n_kmers, ctx->d_K.p, (size_t)nq * 2, host_ptr_pinned(res->n_kmers)));
     CU(d2h(ctx, res->global_signal, ctx->d_global.p, (size_t)nq * 8, host_ptr_pinned(res->global_signal)));
+    if (both) {
+        ctx->h_strand.resize(nq);
+        CU(d2h(ctx, ctx->h_strand.data(), ctx->d_strand.p, nq, false));
+        ctx->prof.d2h_bytes += nq;
+    }
     CU(d2h_finish(ctx));
     const unsigned long long used = ctx->merged ? (unsigned long long)h_begin[nq] : h_used[0], hits = h_used[1];
     ctx->prof.d2h_bytes += 16 + 4 + (u64)nq * (3 * 4 + 2 + 8);
@@ -1376,6 +1457,16 @@ RTX_API int rtx_batch_download(rtx_ctx* ctx, rtx_results* res) {
         ctx->prof.d2h_bytes += (u64)nq * Ns * 2;
     }
     CU(cudaStreamSynchronize(cs));
+    ctx->strands_ready = both;
+    return RTX_OK;
+}
+
+RTX_API int rtx_batch_strands(rtx_ctx* ctx, uint8_t* strand) {
+    if (!ctx) return RTX_ERR_INVALID;
+    REQUIRE(strand != nullptr, "rtx_batch_strands: strand is NULL");
+    REQUIRE(ctx->has_batch && (ctx->bv.flags & RTX_BOTH_STRANDS), "rtx_batch_strands: the batch was not uploaded with RTX_BOTH_STRANDS");
+    REQUIRE(ctx->strands_ready || ctx->bv.n_queries == 0, "rtx_batch_strands: the batch's results were not downloaded yet");
+    if (ctx->bv.n_queries) memcpy(strand, ctx->h_strand.data(), ctx->bv.n_queries);
     return RTX_OK;
 }
 
@@ -1406,7 +1497,11 @@ static int shard_precheck(rtx_ctx* ctx, int want_phase, const char* who) {
     return RTX_OK;
 }
 
+static const char* kNoShardStrands = ": --strand both (RTX_BOTH_STRANDS) is not available in reference-sharded mode";
+
 RTX_API int rtx_shard_phase1(rtx_ctx* ctx) {
+    if (ctx && ctx->has_batch && (ctx->bv.flags & RTX_BOTH_STRANDS))
+        return set_err(ctx, RTX_ERR_UNSUPPORTED, std::string("rtx_shard_phase1") + kNoShardStrands);
     int rc = shard_precheck(ctx, 0, "rtx_shard_phase1");
     if (rc) return rc;
     BatchView& bv = ctx->bv;
@@ -1461,7 +1556,7 @@ RTX_API int rtx_shard_phase2(rtx_ctx* ctx) {
     const u32 nq = bv.n_queries;
     ctx->shard_phase = 2;
     if (nq == 0) return RTX_OK;
-    rc = launch_prob(ctx, 0, (int)nq);
+    rc = launch_prob(ctx, ctx->bv, 0, (int)nq);
     if (rc) return rc;
     if (ctx->sv.n_strad) {
         const long long warps = (long long)nq * ctx->sv.n_strad;
@@ -1494,7 +1589,7 @@ RTX_API int rtx_shard_phase3(rtx_ctx* ctx) {
         shard_combine_kernel<<<(nq + 127) / 128, 128, 0, ctx->stream>>>(ctx->sv, ctx->d_recs.as<NodeRec>(), (int)nq);
         CU(cudaGetLastError());
     }
-    rc = launch_walk<true>(ctx, ctx->sv, ctx->sc, 0, (int)nq, ctx->stream);
+    rc = launch_walk<true>(ctx, ctx->bv, ctx->sv, ctx->sc, 0, (int)nq, ctx->stream);
     if (rc) return rc;
     ctx->cur_stream = ctx->stream;
     rc = order_results(ctx);
@@ -1632,6 +1727,8 @@ static int comm_precheck(rtx_ctx* ctx, const char* who) {
 // own choices) that alternate between two scratch slots: hit counting of sub-batch i+1 runs on `stream` while the histogram
 // all-reduce, the probability / prefix / record kernels, the record all-gather and the tree walk of sub-batch i run on `stream2`.
 RTX_API int rtx_shard_run(rtx_ctx* ctx) {
+    if (ctx && ctx->has_batch && (ctx->bv.flags & RTX_BOTH_STRANDS))
+        return set_err(ctx, RTX_ERR_UNSUPPORTED, std::string("rtx_shard_run") + kNoShardStrands);
     int rc = comm_precheck(ctx, "rtx_shard_run");
     if (rc) return rc;
     CU(cudaSetDevice(ctx->device));
@@ -1705,7 +1802,7 @@ RTX_API int rtx_shard_run(rtx_ctx* ctx) {
             NC(nccl().AllReduce(h, h, (size_t)qb * bv.hstride, ncclUint32, ncclSum, comm, st));
             ctx->prof.allreduce_bytes += (u64)qb * bv.hstride * 4;
         }
-        rc = launch_prob(ctx, (int)q0, qb);
+        rc = launch_prob(ctx, ctx->bv, (int)q0, qb);
         if (rc) return rc;
         ShardView sv = ctx->sv;
         sv.send = ctx->d_send_s[slot].as<ShardRec>();
@@ -1731,7 +1828,7 @@ RTX_API int rtx_shard_run(rtx_ctx* ctx) {
                 CU(cudaGetLastError());
             }
         }
-        rc = launch_walk<true>(ctx, sv, *ctx->cur_sc, (int)q0, qb, st);
+        rc = launch_walk<true>(ctx, ctx->bv, sv, *ctx->cur_sc, (int)q0, qb, st);
         if (rc) return rc;
         if (pipe) CU(cudaEventRecord(ctx->ev_post[slot], ctx->stream2));
     }
@@ -1872,6 +1969,7 @@ RTX_API int rtx_shard_gather(rtx_ctx* ctx, int root) {
 RTX_API int rtx_shard_classify(rtx_ctx* ctx, const rtx_batch* batch, rtx_results* results, int root) {
     if (!ctx) return RTX_ERR_INVALID;
     REQUIRE(results != nullptr, "results is NULL");
+    if (batch && (batch->flags & RTX_BOTH_STRANDS)) return set_err(ctx, RTX_ERR_UNSUPPORTED, std::string("rtx_shard_classify") + kNoShardStrands);
     int rc = rtx_batch_upload(ctx, batch);
     if (rc == RTX_OK) rc = rtx_shard_run(ctx);
     if (rc == RTX_OK) rc = rtx_shard_gather(ctx, root);

@@ -3,6 +3,7 @@
 // Mirrors the reference's CLI surface, output files and restart behaviour (src/io.rs:112-300, src/main.rs:14-173):
 //   raxtax -d <db.fasta[.gz] | db.bin> -i <queries.fasta[.gz]> [-o PREFIX] [--skip-exact-matches] [--raw-confidence] [--tsv]
 //          [--redo] [--only-db] [--skip-db] [-c] [-t N] [--pin] [-v|-q] [--gpu N] [--gpus N [--shard-references]] [--batch N]
+//          [--strand plus|both]
 // writes <PREFIX>/raxtax.out, raxtax.log, raxtax.ckp, raxtax.json and (with --tsv) raxtax.tsv in the reference's formats
 // (lineage.rs:17-48), and <PREFIX>/<database stem>.bin, the bincode database of tree.rs:146-164, unless --skip-db.
 // A database path that deserialises as such a .bin is loaded instead of parsed (parser.rs:37-44).  An interrupted run is
@@ -35,7 +36,7 @@ enum { EX_OK_ = 0, EX_USAGE_ = 64, EX_NOINPUT_ = 66, EX_CANTCREAT_ = 73, EX_IOER
 struct Args {
     std::string database_path, query_file, prefix = "raxtax";
     bool skip_exact_matches = false, tsv = false, only_db = false, skip_db = false, clean = false, raw_confidence = false, redo = false,
-         pin = false, shard_refs = false;
+         pin = false, shard_refs = false, both_strands = false;
     int threads = 0, verbosity = 3 /* Info */, gpu = 0, gpus = 1;
     size_t batch = 0;
 };
@@ -62,6 +63,8 @@ void usage() {
             "      --shard-references               With --gpus N: every GPU holds 1/N of the references (databases too large to\n"
             "                                       replicate) instead of the whole index\n"
             "      --batch <N>                      Queries per device batch [default: all]\n"
+            "      --strand <STRAND>                plus: classify the queries as given; both: in the orientation that shares more\n"
+            "                                       8-mers with some reference, strand column +/- in the outputs [default: plus]\n"
             "  -v, --verbose...                     Increase logging verbosity (repeatable: -vv)\n"
             "  -q, --quiet...                       Decrease logging verbosity (repeatable: -qq)\n");
 }
@@ -169,6 +172,7 @@ struct Checkpoint {
     std::string checkpoint_file, progress_file;
     Fingerprint db;
     bool raw_confidence = false, skip_exact_matches = false, tsv = false;
+    bool both_strands = false;  // "strand": "both", written only in that mode (a plain run keeps the reference's key set)
     std::set<std::string> processed;  // #[serde(skip)]
 };
 std::string json_escape(const std::string& s) {
@@ -196,9 +200,10 @@ bool checkpoint_save(const Checkpoint& c) {  // Checkpoint::save (io.rs:72-78): 
     if (!f) return false;
     fprintf(f,
             "{\n  \"checkpoint_file\": \"%s\",\n  \"progress_file\": \"%s\",\n  \"db_fingerprint\": {\n    \"path\": \"%s\",\n"
-            "    \"size\": %llu,\n    \"modified\": %llu\n  },\n  \"raw_confidence\": %s,\n  \"skip_exact_matches\": %s,\n  \"tsv\": %s\n}",
+            "    \"size\": %llu,\n    \"modified\": %llu\n  },\n  \"raw_confidence\": %s,\n  \"skip_exact_matches\": %s,\n  \"tsv\": %s%s\n}",
             json_escape(c.checkpoint_file).c_str(), json_escape(c.progress_file).c_str(), json_escape(c.db.path).c_str(), c.db.size,
-            c.db.modified, c.raw_confidence ? "true" : "false", c.skip_exact_matches ? "true" : "false", c.tsv ? "true" : "false");
+            c.db.modified, c.raw_confidence ? "true" : "false", c.skip_exact_matches ? "true" : "false", c.tsv ? "true" : "false",
+            c.both_strands ? ",\n  \"strand\": \"both\"" : "");
     if (fclose(f) != 0) return false;
     return rename(tmp.c_str(), c.checkpoint_file.c_str()) == 0;
 }
@@ -276,6 +281,7 @@ bool checkpoint_load(const std::string& path, Checkpoint* c) {  // serde_json::f
     c->db.size = strtoull(v.c_str(), nullptr, 10);
     if (!json_find(j, "modified", &v)) return false;
     c->db.modified = strtoull(v.c_str(), nullptr, 10);
+    c->both_strands = json_find(j, "strand", &v) && v == "both";
     return b("raw_confidence", &c->raw_confidence) && b("skip_exact_matches", &c->skip_exact_matches) && b("tsv", &c->tsv);
 }
 // io::check_incomplete_output (io.rs:156-188): drop the result lines of queries the progress file does not list
@@ -331,6 +337,14 @@ int main(int argc, char** argv) {
         else if (s == "--gpus") a.gpus = std::max(1, atoi(val("--gpus")));
         else if (s == "--shard-references") a.shard_refs = true;
         else if (s == "--batch") a.batch = (size_t)atoll(val("--batch"));
+        else if (s == "--strand") {  // vsearch's spelling
+            const std::string v = val("--strand");
+            if (v != "plus" && v != "both") {
+                fprintf(stderr, "error: invalid value '%s' for '--strand <STRAND>'\n  [possible values: plus, both]\n", v.c_str());
+                return EX_USAGE_;
+            }
+            a.both_strands = v == "both";
+        }
         else if (s == "--verbose") a.verbosity = std::min(5, a.verbosity + 1);  // clap_verbosity_flag::Verbosity<InfoLevel> (io.rs:152-153)
         else if (s == "--quiet") a.verbosity = std::max(0, a.verbosity - 1);
         else if (s.size() >= 2 && s[0] == '-' && s.find_first_not_of('v', 1) == std::string::npos) a.verbosity = std::min(5, a.verbosity + (int)s.size() - 1);  // -v, -vv, ...
@@ -352,6 +366,10 @@ int main(int argc, char** argv) {
         fprintf(stderr, "error: the argument '--only-db' cannot be used with '--skip-db'\n");
         return EX_USAGE_;
     }
+    if (a.both_strands && a.shard_refs) {
+        fprintf(stderr, "error: the argument '--strand both' cannot be used with '--shard-references'\n");
+        return EX_USAGE_;
+    }
     // ---- Args::get_output (io.rs:202-263): checkpoint, output folder, writers ----------------------------------------
     const std::string ckp_path = a.prefix + "/raxtax.json", out_path = a.prefix + "/raxtax.out", tsv_path = a.prefix + "/raxtax.tsv";
     Checkpoint ckp;
@@ -362,6 +380,7 @@ int main(int argc, char** argv) {
         c->raw_confidence = a.raw_confidence;
         c->skip_exact_matches = a.skip_exact_matches;
         c->tsv = a.tsv;
+        c->both_strands = a.both_strands;
         return fingerprint(a.database_path, &c->db);
     };
     bool resumed = false;
@@ -370,7 +389,7 @@ int main(int argc, char** argv) {
         if (checkpoint_load(ckp_path, &old)) {
             Fingerprint now;
             const bool valid = fingerprint(old.db.path, &now) && a.tsv == old.tsv && a.raw_confidence == old.raw_confidence &&
-                               a.skip_exact_matches == old.skip_exact_matches && now == old.db;  // checkpoint_valid (io.rs:288-303)
+                               a.skip_exact_matches == old.skip_exact_matches && a.both_strands == old.both_strands && now == old.db;  // checkpoint_valid (io.rs:288-303)
             if (valid) {
                 std::ifstream prog(old.progress_file);
                 std::string line;
@@ -510,8 +529,8 @@ int main(int argc, char** argv) {
     auto t0 = std::chrono::steady_clock::now();
     int rc = sharded ? rxh_raxtax_sharded(ctxs.data(), ctxs.size(), queries, tree, a.skip_exact_matches, a.raw_confidence, a.batch, send_cb, &w,
                                           a.tsv, log_cb, &w, &warnings)
-                     : rxh_raxtax_multi(ctxs.data(), ctxs.size(), queries, tree, a.skip_exact_matches, a.raw_confidence, a.batch, send_cb, &w,
-                                        a.tsv, log_cb, &w, &warnings);
+                     : (a.both_strands ? rxh_raxtax_both_strands : rxh_raxtax_multi)(ctxs.data(), ctxs.size(), queries, tree, a.skip_exact_matches,
+                                                                                     a.raw_confidence, a.batch, send_cb, &w, a.tsv, log_cb, &w, &warnings);
     double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     if (!w.commit() && rc == 0) {  // the labels still held back: results first, then progress
         fprintf(stderr, "\x1b[31m[ERROR]\x1b[0m Could not write the result files\n");

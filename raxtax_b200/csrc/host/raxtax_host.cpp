@@ -1540,6 +1540,22 @@ struct CharBuf {
     }
 };
 
+// --strand both: the complement of a 4-bit code is its bit-reversed nibble (A1 <-> T8, C2 <-> G4, R5 <-> Y10, N15 <-> N15)
+static inline u8 complement_code(u8 c) {
+    return (u8)(((c & 1u) << 3) | ((c & 2u) << 1) | ((c & 4u) >> 1) | ((c & 8u) >> 3));
+}
+// decompress_sequence of the reverse complement, from the decompressed text ('-' for every ambiguous code stays '-')
+static std::string reverse_complement_text(const std::string& t) {
+    std::string r(t.rbegin(), t.rend());
+    for (char& c : r) c = c == 'A' ? 'T' : c == 'T' ? 'A' : c == 'C' ? 'G' : c == 'G' ? 'C' : c;
+    return r;
+}
+// the strand column of --strand both: `+` classified as given, `-` as the reverse complement
+static inline void strand_column(CharBuf& s, bool minus) {
+    s.put('\t');
+    s.put(minus ? '-' : '+');
+}
+
 static void output_line(CharBuf& s, const std::string& label, const ResultView& r) {  // lineage.rs:17-30
     s.put(label.data(), label.size());
     s.put('\t');
@@ -1637,6 +1653,7 @@ struct ChunkJob {
     std::vector<u32> rep, uniq_first, exact_off, exact_ids;
     std::vector<u64> u_off, uniq_hash;
     std::vector<u8> u_codes;
+    std::vector<u8> rc_seq, strand;  // --strand both: a reverse complement being looked up; per distinct sequence, 1 = classified as rc
     PinnedArr<u16> n_kmers;
     PinnedArr<u32> result_begin, first_ref;
     PinnedArr<double> global, conf, local;
@@ -1757,6 +1774,7 @@ struct Worker {
     Clock t_prep{}, t_issue{}, t_collect{}, t_acquire{}, t_format{}, t_send{}, t_emit_wait{};
     std::chrono::steady_clock::time_point t_start{}, t_first_issue{}, t_last_collect{};
     std::atomic<bool> first_issued{false};
+    bool both = false;  // --strand both (rxh_raxtax_both_strands): RTX_BOTH_STRANDS batches, strand column in both outputs
     static std::chrono::steady_clock::time_point now() { return std::chrono::steady_clock::now(); }
 
     void fail(const std::string& what) {
@@ -1836,11 +1854,31 @@ struct Worker {
                 j.exact_ids.push_back(id);
             j.exact_off[u + 1] = (u32)j.exact_ids.size();
         }
-        if (skip_exact_matches || j.exact_ids.empty() || !log) return;
+        if (both) {  // entries [n, 2n): the exact matches of the reverse complements, the orientation the device may choose instead
+            j.exact_off.resize(2 * j.n_uniq + 1);
+            for (size_t u = 0; u < j.n_uniq; ++u) {
+                const size_t q = c0 + (have_hash ? j.uniq_first[u] : u);
+                const u8* sp = qs.codes.data() + qs.off[q];
+                const size_t sl = (size_t)(qs.off[q + 1] - qs.off[q]);
+                j.rc_seq.resize(sl);
+                for (size_t k = 0; k < sl; ++k) j.rc_seq[k] = complement_code(sp[sl - 1 - k]);
+                const u8* rp = sl ? j.rc_seq.data() : sp;
+                for (u32 id = tree.exact_head(rp, sl, Tree::hash_bytes(rp, sl)); id != Tree::kNone; id = tree.ex_next[id]) j.exact_ids.push_back(id);
+                j.exact_off[j.n_uniq + u + 1] = (u32)j.exact_ids.size();
+            }
+            return;  // the log lines are those of the classified orientation: written after collect (log_exact)
+        }
+        if (log) log_exact(j);
+    }
+
+    // the log lines of raxtax.rs:43-53, per query of the job; with --strand both for the orientation each query was classified in
+    void log_exact(const ChunkJob& j) {
+        if (skip_exact_matches || j.exact_ids.empty()) return;
         std::string msg, first_parent;
-        for (size_t i = 0; i < cn; ++i) {  // the log lines of raxtax.rs:43-53, per query
-            const size_t q = c0 + i;
-            const u32 e0 = j.exact_off[j.rep[i]], e1 = j.exact_off[j.rep[i] + 1];
+        for (size_t i = 0; i < j.cn; ++i) {
+            const size_t q = j.c0 + i;
+            const size_t s = both && j.strand[j.rep[i]] ? j.n_uniq + j.rep[i] : j.rep[i];
+            const u32 e0 = j.exact_off[s], e1 = j.exact_off[s + 1];
             bool all_equal = true;
             for (u32 e = e0; e < e1; ++e) {
                 const std::string& l = tree.lineages[j.exact_ids[e]];
@@ -1875,7 +1913,7 @@ struct Worker {
         batch.seq_codes = j.compact ? j.u_codes.data() : qs.codes.data();
         batch.exact_offsets = j.exact_off.data();
         batch.exact_ids = j.exact_ids.empty() ? nullptr : j.exact_ids.data();
-        batch.flags = (skip_exact_matches ? RTX_SKIP_EXACT_MATCHES : 0u) | (raw_confidence ? RTX_RAW_CONFIDENCE : 0u);
+        batch.flags = (skip_exact_matches ? RTX_SKIP_EXACT_MATCHES : 0u) | (raw_confidence ? RTX_RAW_CONFIDENCE : 0u) | (both ? RTX_BOTH_STRANDS : 0u);
         j.dev_slot = dev_slot;
         if (rtx_batch_slot(ctx, dev_slot)) throw Error(std::string("rtx_batch_slot: ") + rtx_last_error(ctx));
         int rc = rtx_batch_upload(ctx, &batch);
@@ -1919,6 +1957,11 @@ struct Worker {
             }
             if (rc) throw Error(std::string("rtx_batch_download: ") + rtx_last_error(ctx));
             break;
+        }
+        if (both) {
+            j.strand.resize(std::max<size_t>(j.n_uniq, 1));
+            if (rtx_batch_strands(ctx, j.strand.data())) throw Error(std::string("rtx_batch_strands: ") + rtx_last_error(ctx));
+            log_exact(j);
         }
     }
 
@@ -2094,20 +2137,24 @@ struct Worker {
             const size_t q = j.c0 + i;
             const u32 u = j.rep[i];
             const u32 r0 = j.result_begin.p[u], r1 = j.result_begin.p[u + 1];
+            const bool minus = both && j.strand[u];
             out.off.push_back(out.buf.n);
             for (u32 r = r0; r < r1; ++r) {
                 const ResultView rv{&tree.lineages[j.first_ref.p[r]], j.conf.p + (size_t)r * ML, j.n_levels.p[r], j.local.p[r], j.global.p[u]};
                 if (r != r0) out.buf.put('\n');
                 output_line(out.buf, qs.labels[q], rv);
+                if (both) strand_column(out.buf, minus);
             }
             out.buf.put('\0');
             out.off.push_back(out.buf.n);
             if (tsv) {
                 seq = decompress_sequence(qs.codes.data() + qs.off[q], (size_t)(qs.off[q + 1] - qs.off[q]));
+                if (minus) seq = reverse_complement_text(seq);  // the sequence in the orientation that was classified
                 for (u32 r = r0; r < r1; ++r) {
                     const ResultView rv{&tree.lineages[j.first_ref.p[r]], j.conf.p + (size_t)r * ML, j.n_levels.p[r], j.local.p[r], j.global.p[u]};
                     if (r != r0) out.buf.put('\n');
                     tsv_line(out.buf, qs.labels[q], rv, seq);
+                    if (both) strand_column(out.buf, minus);
                 }
                 out.buf.put('\0');
             }
@@ -2286,12 +2333,12 @@ RXH_API size_t rxh_plan_chunks(size_t n_queries, size_t n_ctx, size_t chunk_size
     return b.size();
 }
 
-RXH_API int rxh_raxtax_multi(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queries* queries, const rxh_tree* tree_h, int skip_exact_matches,
-                             int raw_confidence, size_t chunk_size, rxh_sender sender, void* sender_user, int tsv, rxh_logger logger,
-                             void* logger_user, int* warnings) {
+static int raxtax_query_partitioned(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queries* queries, const rxh_tree* tree_h, int skip_exact_matches,
+                                    int raw_confidence, size_t chunk_size, rxh_sender sender, void* sender_user, int tsv, rxh_logger logger,
+                                    void* logger_user, int* warnings, int both_strands, const char* who) {
     if (warnings) *warnings = 0;
     if (!ctxs || n_ctx == 0 || !queries || !tree_h) {
-        g_err = "rxh_raxtax_multi: no context";
+        g_err = std::string(who) + ": no context";
         return -1;
     }
     const size_t nq = queries->q->size();
@@ -2299,6 +2346,7 @@ RXH_API int rxh_raxtax_multi(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queri
     if (chunk_size == 0) chunk_size = default_chunk_size(nq, n_ctx);
     Worker w{*tree_h->t, *queries->q, nq, chunk_size, skip_exact_matches, raw_confidence, tsv, sender, sender_user, logger, logger_user};
     w.ramp = ramp;
+    w.both = both_strands != 0;
     w.run(ctxs, n_ctx);
     if (warnings) *warnings = w.warned.load() ? 1 : 0;
     if (w.failed.load()) {
@@ -2306,6 +2354,20 @@ RXH_API int rxh_raxtax_multi(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queri
         return -1;
     }
     return 0;
+}
+
+RXH_API int rxh_raxtax_multi(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queries* queries, const rxh_tree* tree_h, int skip_exact_matches,
+                             int raw_confidence, size_t chunk_size, rxh_sender sender, void* sender_user, int tsv, rxh_logger logger,
+                             void* logger_user, int* warnings) {
+    return raxtax_query_partitioned(ctxs, n_ctx, queries, tree_h, skip_exact_matches, raw_confidence, chunk_size, sender, sender_user, tsv, logger,
+                                    logger_user, warnings, 0, "rxh_raxtax_multi");
+}
+
+RXH_API int rxh_raxtax_both_strands(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queries* queries, const rxh_tree* tree_h, int skip_exact_matches,
+                                    int raw_confidence, size_t chunk_size, rxh_sender sender, void* sender_user, int tsv, rxh_logger logger,
+                                    void* logger_user, int* warnings) {
+    return raxtax_query_partitioned(ctxs, n_ctx, queries, tree_h, skip_exact_matches, raw_confidence, chunk_size, sender, sender_user, tsv, logger,
+                                    logger_user, warnings, 1, "rxh_raxtax_both_strands");
 }
 
 // Reference-sharded mode: the result lines the ranks emitted for one batch, merged per query.  Lines are ordered like

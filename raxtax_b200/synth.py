@@ -329,6 +329,31 @@ def generate(name="c2", n_refs=None, n_queries=None, length=None, kind=None, see
     return ds
 
 
+# complement of a 4-bit code: the bit-reversed nibble (A1 <-> T8, C2 <-> G4, R5 <-> Y10, N15 <-> N15, ...)
+COMPLEMENT = np.array([int(f"{c:04b}"[::-1], 2) for c in range(16)], np.uint8)
+
+
+def reverse_complement(codes: np.ndarray) -> np.ndarray:
+    """Reverse complement of one sequence of 4-bit codes."""
+    return COMPLEMENT[np.asarray(codes, np.uint8)[::-1] & 15]
+
+
+def reverse_complement_batch(off: np.ndarray, codes: np.ndarray, which=None) -> np.ndarray:
+    """Packed sequences (codes[off[i]:off[i+1]]) with sequence i reverse-complemented where which[i] (all of them when which is
+    None); the offsets do not change."""
+    off = np.asarray(off, np.int64)
+    codes = np.asarray(codes, np.uint8)
+    n = len(off) - 1
+    lens = off[1:] - off[:-1]
+    sel = np.ones(n, bool) if which is None else np.asarray(which, bool)
+    seg = np.repeat(np.arange(n), lens)
+    pos = np.arange(len(codes), dtype=np.int64)
+    flip = sel[seg]
+    src = np.where(flip, off[:-1][seg] + off[1:][seg] - 1 - pos, pos)
+    out = codes[src]
+    return np.where(flip, COMPLEMENT[out & 15], out).astype(np.uint8)
+
+
 def kmers_of(codes: np.ndarray) -> np.ndarray:
     """Sorted unique 8-mers of one sequence of 4-bit codes (utils.rs:27-40), numpy restatement used for data statistics."""
     if len(codes) < 8:
