@@ -70,8 +70,10 @@ typedef enum {
     RTX_OPT_PIPELINE = 11,          /* 1: batches of >= 4096 queries are cut into >= 4 sub-batches and hit counting of sub-batch i+1 overlaps
                                        probabilities / prefix sums / tree walk of sub-batch i on a second, higher-priority stream;
                                        0 (default) = serial: on B200 the overlap only recovers what the shorter launches lose */
-    RTX_OPT_WALK_LOG_CAP = 10       /* test hook: significant-node log capacity of the level-synchronous walk (0 = full); queries that
+    RTX_OPT_WALK_LOG_CAP = 10,      /* test hook: significant-node log capacity of the level-synchronous walk (0 = full); queries that
                                        exceed it take the depth-first retry path */
+    RTX_OPT_BEST_HITS = 12          /* T in 0..64 (0 = off, the default), taken by the next rtx_batch_upload / rtx_classify_batch: each
+                                       query's best hits, read with rtx_batch_best_hits.  Not available in reference-sharded mode */
 } rtx_option;
 
 /* ---- context ------------------------------------------------------------------------------------------- */
@@ -201,6 +203,13 @@ int rtx_batch_slot(rtx_ctx* ctx, int slot);
 /* Orientation each query of a RTX_BOTH_STRANDS batch was classified in: strand[q] = 0 as given, 1 reverse complement.  Valid after
  * rtx_batch_download (or rtx_classify_batch) of such a batch in the active slot; RTX_ERR_INVALID otherwise. */
 int rtx_batch_strands(rtx_ctx* ctx, uint8_t* strand /* [n_queries] */);
+/* Best hits of a batch uploaded with RTX_OPT_BEST_HITS = T > 0: the references r with count[r] >= 1 (the final count row, after the skip
+ * zeroing; with RTX_BOTH_STRANDS of the classified orientation), ordered by count descending, then reference id ascending; the first
+ * n_hits[q] = min(T, #{r : count[r] >= 1}) of them are ref[q * T + i] (ids as rtx_results.first_ref: positions in Tree.lineages) with
+ * count[q * T + i] shared 8-mers.  Entries past n_hits[q] are unspecified.  Valid after rtx_batch_download (or rtx_classify_batch) of
+ * such a batch in the active slot; RTX_ERR_INVALID otherwise. */
+int rtx_batch_best_hits(rtx_ctx* ctx, uint32_t* n_hits /* [n_queries] */, uint32_t* ref /* [n_queries * T] */,
+                        uint16_t* count /* [n_queries * T] */);
 
 /* ---- reference-sharded mode (north_star: NCCL all-reduce of the per-query count histograms) -------------
  * Every rank uploads the same batch.  Per batch (which must fit one sub-batch):
@@ -258,7 +267,8 @@ typedef struct {
 
 /* RTX_K_HITCOUNT counts both passes of a RTX_BOTH_STRANDS batch; RTX_K_FIXUP the skip-exact fix-up of either strand and, with
  * RTX_BOTH_STRANDS, the strand decision behind it (strand_select_kernel: M of both strands, the winners' rows copied over the query's;
- * strand_exact_kernel: the exact-match lists of the classified orientations) */
+ * strand_exact_kernel: the exact-match lists of the classified orientations); RTX_K_PREFIX also the best-hits selection of a batch
+ * with RTX_OPT_BEST_HITS > 0 (best_hits_kernel) */
 enum { RTX_K_KMERS = 0, RTX_K_HITCOUNT = 1, RTX_K_FIXUP = 2, RTX_K_PROB = 3, RTX_K_INDEX = 4, RTX_K_WALK = 5, RTX_K_PREFIX = 6,
        RTX_K_ALLREDUCE = 7 /* histogram all-reduce */, RTX_K_ALLGATHER = 8 /* straddler records, result offsets */,
        RTX_K_SHARD = 9 /* record / combine / merge kernels */, RTX_K_GATHER = 10 /* result lines -> root */, RTX_K_COUNT = 11 };

@@ -130,6 +130,17 @@ int rxh_raxtax_both_strands(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_querie
                             int raw_confidence, size_t chunk_size, rxh_sender sender, void* sender_user, int tsv, rxh_logger logger,
                             void* logger_user, int* warnings);
 
+/* rxh_raxtax_multi (both_strands = 0) or rxh_raxtax_both_strands (1) that also reports each query's best hits (RTX_OPT_BEST_HITS =
+ * best_hits, 1..64; 0 = none and hits_sender is never called): hits_sender(hits_user, query_label, hit_lines) is called right before the
+ * query's sender, on the same thread.  hit_lines holds one line per hit, '\n'-separated, without a final newline, empty for a query
+ * without hits: `{label}\t{rank 1..}\t{lineage}\t{shared 8-mers}\t{K}\t{reference id}`, with both_strands followed by the strand column
+ * (`\t+` / `\t-`).  Reference ids are positions in Tree.lineages.  Not available over a reference-sharded index. */
+typedef int (*rxh_hits_sender)(void* user, const char* query_label, const char* hit_lines);
+int rxh_raxtax_best_hits(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queries* queries, const rxh_tree* tree, int skip_exact_matches,
+                         int raw_confidence, size_t chunk_size, rxh_sender sender, void* sender_user, int tsv, rxh_logger logger,
+                         void* logger_user, int* warnings, int both_strands, uint32_t best_hits, rxh_hits_sender hits_sender,
+                         void* hits_user);
+
 /* raxtax::raxtax over a reference-sharded index (BASELINE config 5: databases too large to replicate) with all shards driven by this
  * process: ctxs[r] holds shard r of n_ctx (rxh_tree_upload_sharded).  When every shard sits on its own GPU the contexts are joined into
  * an NCCL communicator and one driver thread per rank calls rtx_shard_run / rtx_shard_gather (histogram all-reduce, record all-gather

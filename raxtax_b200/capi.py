@@ -22,7 +22,7 @@ RTX_OK, RTX_ERR_INVALID, RTX_ERR_CUDA, RTX_ERR_NO_DEVICE, RTX_ERR_NO_INDEX, RTX_
 RTX_SKIP_EXACT_MATCHES, RTX_RAW_CONFIDENCE, RTX_BOTH_STRANDS = 1, 2, 4
 RTX_HITCOUNT_BITROWS, RTX_HITCOUNT_CSR = 0, 1
 RTX_OPT_HITCOUNT_VARIANT, RTX_OPT_SUB_BATCH, RTX_OPT_KEEP_CSR, RTX_OPT_PROFILE, RTX_OPT_HITCOUNT_MAX_TILES = 1, 2, 3, 4, 6
-RTX_OPT_HITCOUNT_GROUP, RTX_OPT_WALK_VARIANT, RTX_OPT_WALK_LOG_CAP, RTX_OPT_PIPELINE = 7, 9, 10, 11
+RTX_OPT_HITCOUNT_GROUP, RTX_OPT_WALK_VARIANT, RTX_OPT_WALK_LOG_CAP, RTX_OPT_PIPELINE, RTX_OPT_BEST_HITS = 7, 9, 10, 11, 12
 KERNEL_NAMES = ["kmers", "hitcount", "fixup", "prob", "index", "walk", "prefix", "allreduce", "allgather", "shard", "gather"]
 
 # every symbol include/raxtax_b200.h declares
@@ -30,7 +30,7 @@ DEVICE_SYMBOLS = [
     "rtx_abi_version", "rtx_ctx_create", "rtx_ctx_destroy", "rtx_last_error", "rtx_ctx_set_option", "rtx_ctx_stream", "rtx_ctx_device",
     "rtx_ctx_synchronize", "rtx_host_alloc", "rtx_host_free", "rtx_index_upload", "rtx_index_n_refs", "rtx_index_shard_refs", "rtx_index_max_levels", "rtx_batch_sub_batch",
     "rtx_index_device_bytes", "rtx_index_bitrow_bytes", "rtx_hitcount_kernel_name", "rtx_classify_batch", "rtx_batch_upload", "rtx_batch_run", "rtx_batch_download", "rtx_batch_slot",
-    "rtx_batch_strands",
+    "rtx_batch_strands", "rtx_batch_best_hits",
     "rtx_shard_phase1", "rtx_shard_hist_buffer", "rtx_shard_phase2", "rtx_shard_records_buffers", "rtx_shard_phase3", "rtx_shard_exchange_hist_local", "rtx_shard_exchange_records_local",
     "rtx_comm_unique_id", "rtx_comm_init", "rtx_comm_destroy", "rtx_shard_run", "rtx_shard_gather", "rtx_shard_classify",
     "rtx_profile_reset", "rtx_profile_get",
@@ -39,7 +39,7 @@ DEVICE_SYMBOLS = [
 HOST_SYMBOLS = [
     "rxh_last_error", "rxh_tree_from_fasta", "rxh_tree_from_file", "rxh_queries_from_file", "rxh_tree_from_bin", "rxh_tree_save_bin", "rxh_queries_skip", "rxh_tree_new", "rxh_tree_free", "rxh_tree_num_tips", "rxh_tree_lineage",
     "rxh_tree_csr", "rxh_tree_build_kmer_map", "rxh_tree_has_kmer_map", "rxh_tree_exact", "rxh_tree_index_desc", "rxh_tree_upload", "rxh_tree_upload_sharded", "rxh_queries_from_fasta", "rxh_queries_new",
-    "rxh_queries_free", "rxh_queries_len", "rxh_queries_label", "rxh_queries_arrays", "rxh_raxtax", "rxh_raxtax_multi", "rxh_raxtax_both_strands", "rxh_raxtax_sharded", "rxh_merge_shard_results", "rxh_exact_batch", "rxh_count_sender", "rxh_count_logger", "rxh_format_fixed", "rxh_release_buffers", "rxh_plan_chunks",
+    "rxh_queries_free", "rxh_queries_len", "rxh_queries_label", "rxh_queries_arrays", "rxh_raxtax", "rxh_raxtax_multi", "rxh_raxtax_both_strands", "rxh_raxtax_best_hits", "rxh_raxtax_sharded", "rxh_merge_shard_results", "rxh_exact_batch", "rxh_count_sender", "rxh_count_logger", "rxh_format_fixed", "rxh_release_buffers", "rxh_plan_chunks",
 ]
 
 
@@ -74,6 +74,7 @@ class Profile(C.Structure):
 
 SENDER = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_char_p, C.c_char_p, C.c_char_p)
 LOGGER = C.CFUNCTYPE(None, C.c_void_p, C.c_int, C.c_char_p)
+HITS_SENDER = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_char_p, C.c_char_p)
 
 _dev = None
 _host = None
@@ -122,6 +123,7 @@ def device_lib():
     L.rtx_batch_slot.argtypes = [C.c_void_p, C.c_int]
     L.rtx_batch_download.argtypes = [C.c_void_p, C.POINTER(ResultsStruct)]
     L.rtx_batch_strands.argtypes = [C.c_void_p, u8p]
+    L.rtx_batch_best_hits.argtypes = [C.c_void_p, u32p, u32p, u16p]
     for f in ("rtx_shard_phase1", "rtx_shard_phase2", "rtx_shard_phase3", "rtx_profile_reset"):
         getattr(L, f).argtypes = [C.c_void_p]
     L.rtx_shard_hist_buffer.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]
@@ -196,6 +198,9 @@ def host_lib():
                                    C.c_int, LOGGER, C.c_void_p, C.POINTER(C.c_int)]
     L.rxh_raxtax_both_strands.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, SENDER,
                                           C.c_void_p, C.c_int, LOGGER, C.c_void_p, C.POINTER(C.c_int)]
+    L.rxh_raxtax_best_hits.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, SENDER,
+                                       C.c_void_p, C.c_int, LOGGER, C.c_void_p, C.POINTER(C.c_int), C.c_int, C.c_uint32, HITS_SENDER,
+                                       C.c_void_p]
     L.rxh_raxtax_sharded.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, SENDER, C.c_void_p,
                                      C.c_int, LOGGER, C.c_void_p, C.POINTER(C.c_int)]
     L.rxh_merge_shard_results.argtypes = [C.c_size_t, C.c_size_t, C.c_uint32, C.POINTER(u32p), C.POINTER(u32p), C.POINTER(u8p), C.POINTER(f64p),
@@ -239,6 +244,8 @@ class ClassifyOutput:
     kmers: np.ndarray | None = None
     probs: np.ndarray | None = None  # [nq, kmax + 1] normalised P(m) by count (valid where the histogram is non-zero)
     strand: np.ndarray | None = None  # both-strand batches: u8 [nq], 0 = classified as given, 1 = as its reverse complement
+    # batches with best_hits = T > 0: (n_hits u32 [nq], ref u32 [nq, T], count u16 [nq, T]); row q is valid up to n_hits[q]
+    best_hits: tuple | None = None
 
     def for_query(self, q):
         a, b = int(self.result_begin[q]), int(self.result_begin[q + 1])
@@ -474,14 +481,32 @@ class Context:
         self._check(device_lib().rtx_batch_strands(self._h, _ptr(s, C.c_uint8)))
         return s[:nq]
 
+    def batch_best_hits(self, nq):
+        """rtx_batch_best_hits of the downloaded batch in the active slot: (n_hits [nq], ref [nq, T], count [nq, T]), the references
+        with the most shared 8-mers by count descending, then id ascending; entries of row q past n_hits[q] are unspecified."""
+        T = max(getattr(self, "_best_hits", {}).get(getattr(self, "_slot", 0), 0), 1)
+        n = np.zeros(max(nq, 1), np.uint32)
+        ref = np.zeros((max(nq, 1), T), np.uint32)
+        cnt = np.zeros((max(nq, 1), T), np.uint16)
+        self._check(device_lib().rtx_batch_best_hits(self._h, _ptr(n, C.c_uint32), _ptr(ref, C.c_uint32), _ptr(cnt, C.c_uint16)))
+        return n[:nq], ref[:nq], cnt[:nq]
+
+    def _set_best_hits(self, best_hits):
+        self.set_option(RTX_OPT_BEST_HITS, best_hits)
+        if not hasattr(self, "_best_hits"):
+            self._best_hits = {}
+        self._best_hits[getattr(self, "_slot", 0)] = int(best_hits)
+
     def classify(self, seq_off, codes, exact_off=None, exact_ids=None, skip_exact=False, raw_conf=False, taps=(), out=None, shard_root=None,
-                 both_strands=False) -> ClassifyOutput:
+                 both_strands=False, best_hits=0) -> ClassifyOutput:
         """rtx_classify_batch: H2D + kernels + D2H in one call.  out = pinned_results(...) reuses page-locked result buffers.
         shard_root = r: rtx_shard_classify instead (reference-sharded mode over NCCL, every rank calls it with the same batch; the
         final lines come back on rank r, nothing on the others).  both_strands: every query is classified in the orientation that
         shares more 8-mers with some reference (RTX_BOTH_STRANDS); exact_off then has 2n + 1 entries (Tree.exact_batch_both_strands)
-        and the result's .strand tells the orientation."""
+        and the result's .strand tells the orientation.  best_hits = T in 1..64: the result's .best_hits holds each query's T best
+        hits (RTX_OPT_BEST_HITS, batch_best_hits)."""
         L = device_lib()
+        self._set_best_hits(best_hits)
         flags = self._flags(skip_exact, raw_conf, both_strands)
         b, keep = self._make_batch(seq_off, codes, exact_off, exact_ids, flags)
         nq = b.n_queries
@@ -508,9 +533,12 @@ class Context:
             self._check(rc)
             if both_strands:
                 out.strand = self.batch_strands(nq)
+            if best_hits:
+                out.best_hits = self.batch_best_hits(nq)
             return self._trim(out, int(r.n_results))
 
-    def batch_upload(self, seq_off, codes, exact_off=None, exact_ids=None, skip_exact=False, raw_conf=False, both_strands=False):
+    def batch_upload(self, seq_off, codes, exact_off=None, exact_ids=None, skip_exact=False, raw_conf=False, both_strands=False, best_hits=0):
+        self._set_best_hits(best_hits)
         flags = self._flags(skip_exact, raw_conf, both_strands)
         b, keep = self._make_batch(seq_off, codes, exact_off, exact_ids, flags)
         self._check(device_lib().rtx_batch_upload(self._h, C.byref(b)))
@@ -536,6 +564,8 @@ class Context:
             self._check(rc)
             if both_strands:
                 out.strand = self.batch_strands(nq)
+            if self._best_hits.get(getattr(self, "_slot", 0), 0):
+                out.best_hits = self.batch_best_hits(nq)
             return self._trim(out, int(r.n_results))
 
     def profile_reset(self):
@@ -776,14 +806,15 @@ class Queries:
 
 
 def raxtax(ctx: Context, queries: Queries, tree: Tree, skip_exact_matches=False, raw_confidence=False, chunk_size=0, tsv=False, sharded=False,
-           both_strands=False):
+           both_strands=False, best_hits=0):
     """raxtax::raxtax (raxtax.rs:14-97).  Returns (results, log_lines, warnings) where results is the list of
     (query_label, primary_results, tsv_results_or_None) tuples the reference sends to its writer thread.  both_strands: every query
     is classified in the orientation that shares more 8-mers with some reference (rxh_raxtax_both_strands, one or several contexts);
-    every line then ends in a strand column (`+` / `-`)."""
-    if both_strands and sharded:
-        raise ValueError("both_strands is not available over a reference-sharded index")
-    sent, logs = [], []
+    every line then ends in a strand column (`+` / `-`).  best_hits = N in 1..64 (rxh_raxtax_best_hits): returns
+    (results, log_lines, warnings, hits) with hits the list of (query_label, hit_lines) in the order the queries were sent."""
+    if (both_strands or best_hits) and sharded:
+        raise ValueError("both_strands and best_hits are not available over a reference-sharded index")
+    sent, logs, hits = [], [], []
 
     def _send(_u, label, primary, tsv_s):
         sent.append((label.decode(), primary.decode(), tsv_s.decode() if tsv_s is not None else None))
@@ -792,8 +823,18 @@ def raxtax(ctx: Context, queries: Queries, tree: Tree, skip_exact_matches=False,
     def _log(_u, level, msg):
         logs.append((level, msg.decode()))
 
+    def _hits(_u, label, lines):
+        hits.append((label.decode(), lines.decode()))
+        return 0
+
     warn = C.c_int(0)
-    if both_strands:
+    if best_hits:
+        ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
+        arr = (C.c_void_p * len(ctxs))(*[c._h for c in ctxs])
+        rc = host_lib().rxh_raxtax_best_hits(arr, len(ctxs), queries._h, tree._h, int(skip_exact_matches), int(raw_confidence), int(chunk_size),
+                                             SENDER(_send), None, int(tsv), LOGGER(_log), None, C.byref(warn), int(both_strands),
+                                             int(best_hits), HITS_SENDER(_hits), None)
+    elif both_strands:
         ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
         arr = (C.c_void_p * len(ctxs))(*[c._h for c in ctxs])
         rc = host_lib().rxh_raxtax_both_strands(arr, len(ctxs), queries._h, tree._h, int(skip_exact_matches), int(raw_confidence), int(chunk_size),
@@ -811,4 +852,6 @@ def raxtax(ctx: Context, queries: Queries, tree: Tree, skip_exact_matches=False,
                                    None, int(tsv), LOGGER(_log), None, C.byref(warn))
     if rc != 0:
         raise _host_err()
+    if best_hits:
+        return sent, logs, bool(warn.value), hits
     return sent, logs, bool(warn.value)

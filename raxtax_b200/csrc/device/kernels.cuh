@@ -9,6 +9,7 @@
 //   K4 prefix_kernel           prefix sums of the probabilities at node boundaries (lineage.rs:61-77,114-117)
 //   K5 lineage_walk_kernel     tree walk with the 0.01 cutoff / fallback (lineage.rs:119-179), signals and ordering
 //                              (lineage.rs:86-111), override (raxtax.rs:73-84)
+//      best_hits_kernel        optional: each query's T references with the most shared 8-mers, from the resident count row
 #pragma once
 
 #include <math_constants.h>
@@ -1419,6 +1420,139 @@ __global__ void __launch_bounds__(kPrefixThreads)
         }
     }
     for (u32 i = tid; i < (n_seg + 31u) / 32u; i += kPrefixThreads) aux[2 + i] = skipw_s[i];
+}
+
+// =========================================================================================================
+// Best hits (RTX_OPT_BEST_HITS = T): the references with count >= 1, by count descending then id ascending, first min(T, #) of
+// them.  One CTA per query of the sub-batch, behind the skip zeroing and the strand decision, while the count row is resident.
+//   1. From the histogram, scanning down from K: tau = the largest m >= 1 with #{c >= m} >= T (1 if fewer than T references have a
+//      hit) and g = #{c > tau} < T.  Exactly the g references above tau and the T - g lowest ids at tau are wanted.
+//   2. Candidate segments (512 references): those whose maximum reaches tau, every one when there are no per-segment maxima.  In skip
+//      mode the maxima were taken before the zeroing and are only upper bounds: they filter, nothing more.
+//   3. The candidates in ascending id order, one warp per segment: every count > tau and the first ties at tau, positions from a
+//      block-ordered prefix.  The histogram is exact, so the scan stops once both targets are met.
+//   4. The < T counts above tau ranked by (count desc, id asc), the ties behind them in id order.
+// =========================================================================================================
+constexpr int kBestThreads = 256;
+constexpr int kBestWarps = kBestThreads / 32;
+constexpr u32 kBestHitsMax = 64;
+
+__global__ void __launch_bounds__(kBestThreads)
+    best_hits_kernel(IndexView ix, BatchView b, ProbScratch sc, const u16* __restrict__ counts, int use_segmax, u32 T, int q_base,
+                     u32* __restrict__ n_hits, u32* __restrict__ hit_ref, u16* __restrict__ hit_count) {
+    __shared__ u32 wsum[kBestWarps];
+    __shared__ u32 s_tau, s_g;
+    __shared__ u32 s_cand[kBestThreads];
+    __shared__ u32 s_above_ref[kBestHitsMax], s_tie_ref[kBestHitsMax];
+    __shared__ u16 s_above_cnt[kBestHitsMax];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int ql = blockIdx.x, q = q_base + ql;
+    const u32 K = b.K[q];
+    const u32* __restrict__ hist = b.hist + (size_t)q * b.hstride;
+    if (tid == 0) s_tau = 0;
+    __syncthreads();
+    // ---- 1. threshold: thread t of a round holds bucket top - t; its exclusive prefix is #{c > m} ------------------------------
+    u32 above = 0;  // #{c > the round's lowest bucket}
+    for (u32 top = K; top > 0; top -= min(top, (u32)kBestThreads)) {
+        const u32 m = top - (u32)tid;
+        const u32 h = (u32)tid < top ? hist[m] : 0u;
+        u32 total;
+        const u32 gt = above + block_scan_excl(h, wsum, tid, kBestWarps, &total);
+        if (h && gt < T && gt + h >= T) {  // the one bucket where #{c >= m} reaches T
+            s_tau = m;
+            s_g = gt;
+        }
+        __syncthreads();
+        if (s_tau) break;
+        above += total;
+    }
+    u32 tau = s_tau, g = s_g;
+    if (tau == 0) {  // fewer than T references with a hit: all of them
+        tau = 1;
+        g = K >= 1 ? above - hist[1] : 0u;
+    }
+    const u32 with_hit = K >= 1 ? (s_tau ? T : above) : 0u;
+    const u32 need_tie = with_hit - g;
+    if (with_hit == 0) {
+        if (tid == 0) n_hits[q] = 0;
+        return;
+    }
+    // ---- 2./3. candidate segments in windows of kBestThreads, then one warp per candidate ----------------------------------------
+    const u32 Ns = (u32)ix.shard_refs;
+    const u32 n_seg = (u32)(ix.n_pad / kPrefixSeg), n_seg_refs = (Ns + kPrefixSeg - 1) / kPrefixSeg;
+    const u16* __restrict__ smax = use_segmax ? seg_max(sc, ql, n_seg) : nullptr;
+    const u16* __restrict__ row = counts + (size_t)ql * ix.n_pad;
+    u32 got_above = 0, got_tie = 0;
+    bool done = false;
+    for (u32 w0 = 0; w0 < n_seg_refs && !done; w0 += kBestThreads) {
+        const u32 s = w0 + (u32)tid;
+        const u32 cand = s < n_seg_refs && (smax == nullptr || (u32)smax[s] >= tau) ? 1u : 0u;
+        u32 n_cand;
+        const u32 slot = block_scan_excl(cand, wsum, tid, kBestWarps, &n_cand);
+        if (cand) s_cand[slot] = s;
+        __syncthreads();
+        for (u32 c0 = 0; c0 < n_cand; c0 += kBestWarps) {
+            const u32 ci = c0 + (u32)warp;
+            u32 r0 = Ns;  // no segment for this warp: every reference reads as past the end
+            uint4 x0 = make_uint4(0, 0, 0, 0), x1 = x0;
+            if (ci < n_cand) {
+                r0 = s_cand[ci] * kPrefixSeg + (u32)lane * 16u;
+                x0 = *reinterpret_cast<const uint4*>(row + r0);
+                x1 = *reinterpret_cast<const uint4*>(row + r0 + 8);
+            }
+            const u32 w[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
+            u32 n_above = 0, n_tie = 0;
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+                const u32 c = r0 + (u32)i < Ns ? (w[i >> 1] >> (16 * (i & 1))) & 0xFFFFu : 0u;
+                n_above += c > tau;
+                n_tie += c == tau;
+            }
+            u32 total;  // both counts packed: at most kBestThreads * 16 per round
+            const u32 ex = block_scan_excl(n_above | n_tie << 16, wsum, tid, kBestWarps, &total);
+            u32 pa = got_above + (ex & 0xFFFFu), pt = got_tie + (ex >> 16);
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+                const u32 c = r0 + (u32)i < Ns ? (w[i >> 1] >> (16 * (i & 1))) & 0xFFFFu : 0u;
+                if (c > tau) {
+                    if (pa < kBestHitsMax) {
+                        s_above_ref[pa] = r0 + (u32)i;
+                        s_above_cnt[pa] = (u16)c;
+                    }
+                    ++pa;
+                } else if (c == tau) {
+                    if (pt < need_tie) s_tie_ref[pt] = r0 + (u32)i;
+                    ++pt;
+                }
+            }
+            got_above += total & 0xFFFFu;
+            got_tie += total >> 16;
+            if (got_above >= g && got_tie >= need_tie) {
+                done = true;
+                break;
+            }
+        }
+    }
+    __syncthreads();
+    // ---- 4. rank the counts above tau; the ties follow in id order -------------------------------------------------------------
+    u32* __restrict__ out_ref = hit_ref + (size_t)q * T;
+    u16* __restrict__ out_cnt = hit_count + (size_t)q * T;
+    const u64 id0 = ix.shard_begin;
+    if ((u32)tid < g) {
+        const u32 c = s_above_cnt[tid], r = s_above_ref[tid];
+        u32 rank = 0;
+        for (u32 j = 0; j < g; ++j) {
+            const u32 cj = s_above_cnt[j];
+            rank += cj > c || (cj == c && s_above_ref[j] < r);
+        }
+        out_ref[rank] = (u32)(id0 + r);
+        out_cnt[rank] = (u16)c;
+    }
+    if ((u32)tid < need_tie) {
+        out_ref[g + tid] = (u32)(id0 + s_tie_ref[tid]);
+        out_cnt[g + tid] = (u16)tau;
+    }
+    if (tid == 0) n_hits[q] = with_hit;
 }
 
 // =========================================================================================================

@@ -64,6 +64,12 @@ struct BatchState {
     DevBuf d_strand, d_sel_off, d_sel_ids;
     std::vector<u8> h_strand;
     bool strands_ready = false;
+    // RTX_OPT_BEST_HITS as the batch was uploaded with (0 = off): per query the hit count, then T reference ids and T counts
+    u32 best_hits = 0;
+    DevBuf d_bh_n, d_bh_ref, d_bh_cnt;
+    std::vector<u32> h_bh_n, h_bh_ref;
+    std::vector<u16> h_bh_cnt;
+    bool hits_ready = false;
     // reference-sharded mode over NCCL
     bool sub_batch_agreed = false;  // the ranks settled on one sub-batch size for this batch
     bool merged = false;            // rtx_shard_gather ran: d_ord_* hold the merged lines (root) / nothing (other ranks)
@@ -97,6 +103,7 @@ struct rtx_ctx : BatchState {
     int walk_variant = 0;  // RTX_OPT_WALK_VARIANT: 0 level-synchronous (+ depth-first retry), 1 depth-first only
     int walk_log_cap = 0;  // RTX_OPT_WALK_LOG_CAP
     int hit_group = 0;   // RTX_OPT_HITCOUNT_GROUP
+    u32 best_hits_opt = 0;  // RTX_OPT_BEST_HITS, taken over by the next rtx_batch_upload
     // index
     bool has_index = false;
     IndexView ix{};
@@ -341,7 +348,7 @@ RTX_API void rtx_ctx_destroy(rtx_ctx* c) {
                         &s.d_pool_first, &s.d_pool_nlev, &s.d_pool_conf, &s.d_pool_local, &s.d_pool_used, &s.d_res_off, &s.d_res_cnt,
                         &s.d_global, &s.d_status, &s.d_hits, &s.d_ord_begin, &s.d_ord_first, &s.d_ord_nlev, &s.d_ord_conf, &s.d_ord_local,
                         &s.d_counts, &s.d_counts1, &s.d_prob_big, &s.d_cbuf, &s.d_preb, &s.d_ptab, &s.d_segoff, &s.d_preb1, &s.d_ptab1, &s.d_segoff1,
-                        &s.d_strand, &s.d_sel_off, &s.d_sel_ids};
+                        &s.d_strand, &s.d_sel_off, &s.d_sel_ids, &s.d_bh_n, &s.d_bh_ref, &s.d_bh_cnt};
         for (DevBuf* b : sb) b->release();
         if (s.ev_up) cudaEventDestroy(s.ev_up);
         if (s.ev_done) cudaEventDestroy(s.ev_done);
@@ -393,6 +400,10 @@ RTX_API int rtx_ctx_set_option(rtx_ctx* ctx, int option, int64_t value) {
         case RTX_OPT_HITCOUNT_GROUP:
             REQUIRE(value >= 0 && value <= kHitGroupMaxThreads / 32, "bad query group size");
             ctx->hit_group = (int)value;
+            return RTX_OK;
+        case RTX_OPT_BEST_HITS:
+            REQUIRE(value >= 0 && value <= (int64_t)kBestHitsMax, "best hits must be in [0, 64]");
+            ctx->best_hits_opt = (u32)value;
             return RTX_OK;
         default:
             return set_err(ctx, RTX_ERR_INVALID, "unknown option");
@@ -815,6 +826,8 @@ RTX_API int rtx_batch_upload(rtx_ctx* ctx, const rtx_batch* batch) {
     ctx->has_batch = false;
     ctx->ran = false;
     ctx->strands_ready = false;
+    ctx->hits_ready = false;
+    ctx->best_hits = ctx->best_hits_opt;
     BatchView& bv = ctx->bv;
     bv = BatchView{};
     bv.n_queries = nq;
@@ -907,6 +920,11 @@ RTX_API int rtx_batch_upload(rtx_ctx* ctx, const rtx_batch* batch) {
             CU(ctx->d_sel_off.ensure(((size_t)nq + 1) * 4));
             CU(ctx->d_sel_ids.ensure(std::max<u64>(total_exact, 1) * 4));
         }
+    }
+    if (ctx->best_hits) {
+        CU(ctx->d_bh_n.ensure((size_t)nq * 4));
+        CU(ctx->d_bh_ref.ensure((size_t)nq * ctx->best_hits * 4));
+        CU(ctx->d_bh_cnt.ensure((size_t)nq * ctx->best_hits * 2));
     }
     bv.K = ctx->d_K.as<u16>();
     bv.kmers = ctx->d_kmers.as<u16>();
@@ -1291,6 +1309,13 @@ static int run_all(rtx_ctx* ctx) {
             int rc2 = launch_walk<false>(ctx, tail, ShardView{}, *ctx->cur_sc, (int)q0, qb, ctx->cur_stream);
             if (rc2) return rc2;
         }
+        if (ctx->best_hits) {  // the count row is still the sub-batch's: K3-K5 only read it, the slot's next tenant waits for ev_post
+            LaunchTimer lt(ctx, RTX_K_PREFIX);
+            best_hits_kernel<<<qb, kBestThreads, 0, ctx->cur_stream>>>(ctx->ix, bv, *ctx->cur_sc, ctx->cur_counts, ctx->segmax_valid ? 1 : 0,
+                                                                        ctx->best_hits, (int)q0, ctx->d_bh_n.as<u32>(),
+                                                                        ctx->d_bh_ref.as<u32>(), ctx->d_bh_cnt.as<u16>());
+            CU(cudaGetLastError());
+        }
         if (ctx->tap_counts_host) {
             const u64 Ns = ctx->ix.shard_refs;
             CU(cudaMemcpy2DAsync(ctx->tap_counts_host + (size_t)q0 * Ns, Ns * 2, ctx->cur_counts, ctx->ix.n_pad * 2, Ns * 2, qb,
@@ -1351,7 +1376,9 @@ RTX_API int rtx_batch_download(rtx_ctx* ctx, rtx_results* res) {
     CU(cudaStreamWaitEvent(cs, ctx->ev_done, 0));  // this slot's kernels; the other slot may be running on `stream` meanwhile
     // round 1: per-query metadata through the pinned arena, one synchronisation
     const bool both = (bv.flags & RTX_BOTH_STRANDS) != 0;
-    const size_t meta_bytes = 2 * 64 + ((size_t)nq + 1) * 4 + (size_t)nq * (4 + 4 + 2 + 8) + 6 * 64 + (both ? (size_t)nq + 64 : 0);
+    const u32 T = ctx->best_hits;
+    const size_t meta_bytes = 2 * 64 + ((size_t)nq + 1) * 4 + (size_t)nq * (4 + 4 + 2 + 8) + 6 * 64 + (both ? (size_t)nq + 64 : 0) +
+                              (T ? (size_t)nq * (4 + (size_t)T * 6) + 3 * 64 : 0);
     CU(arena_reserve(ctx, meta_bytes));
     unsigned long long* h_used = (unsigned long long*)arena_take(ctx, 16);
     u32* h_begin = (u32*)arena_take(ctx, ((size_t)nq + 1) * 4);
@@ -1368,6 +1395,15 @@ RTX_API int rtx_batch_download(rtx_ctx* ctx, rtx_results* res) {
         ctx->h_strand.resize(nq);
         CU(d2h(ctx, ctx->h_strand.data(), ctx->d_strand.p, nq, false));
         ctx->prof.d2h_bytes += nq;
+    }
+    if (T) {
+        ctx->h_bh_n.resize(nq);
+        ctx->h_bh_ref.resize((size_t)nq * T);
+        ctx->h_bh_cnt.resize((size_t)nq * T);
+        CU(d2h(ctx, ctx->h_bh_n.data(), ctx->d_bh_n.p, (size_t)nq * 4, false));
+        CU(d2h(ctx, ctx->h_bh_ref.data(), ctx->d_bh_ref.p, (size_t)nq * T * 4, false));
+        CU(d2h(ctx, ctx->h_bh_cnt.data(), ctx->d_bh_cnt.p, (size_t)nq * T * 2, false));
+        ctx->prof.d2h_bytes += (u64)nq * (4 + (u64)T * 6);
     }
     CU(d2h_finish(ctx));
     const unsigned long long used = ctx->merged ? (unsigned long long)h_begin[nq] : h_used[0], hits = h_used[1];
@@ -1458,6 +1494,7 @@ RTX_API int rtx_batch_download(rtx_ctx* ctx, rtx_results* res) {
     }
     CU(cudaStreamSynchronize(cs));
     ctx->strands_ready = both;
+    ctx->hits_ready = T != 0;
     return RTX_OK;
 }
 
@@ -1467,6 +1504,20 @@ RTX_API int rtx_batch_strands(rtx_ctx* ctx, uint8_t* strand) {
     REQUIRE(ctx->has_batch && (ctx->bv.flags & RTX_BOTH_STRANDS), "rtx_batch_strands: the batch was not uploaded with RTX_BOTH_STRANDS");
     REQUIRE(ctx->strands_ready || ctx->bv.n_queries == 0, "rtx_batch_strands: the batch's results were not downloaded yet");
     if (ctx->bv.n_queries) memcpy(strand, ctx->h_strand.data(), ctx->bv.n_queries);
+    return RTX_OK;
+}
+
+RTX_API int rtx_batch_best_hits(rtx_ctx* ctx, uint32_t* n_hits, uint32_t* ref, uint16_t* count) {
+    if (!ctx) return RTX_ERR_INVALID;
+    REQUIRE(ctx->has_batch && ctx->best_hits, "rtx_batch_best_hits: the batch was not uploaded with RTX_OPT_BEST_HITS > 0");
+    REQUIRE(ctx->hits_ready || ctx->bv.n_queries == 0, "rtx_batch_best_hits: the batch's results were not downloaded yet");
+    const size_t nq = ctx->bv.n_queries, T = ctx->best_hits;
+    REQUIRE(nq == 0 || (n_hits && ref && count), "rtx_batch_best_hits: n_hits / ref / count is NULL");
+    if (nq) {
+        memcpy(n_hits, ctx->h_bh_n.data(), nq * 4);
+        memcpy(ref, ctx->h_bh_ref.data(), nq * T * 4);
+        memcpy(count, ctx->h_bh_cnt.data(), nq * T * 2);
+    }
     return RTX_OK;
 }
 
@@ -1498,10 +1549,13 @@ static int shard_precheck(rtx_ctx* ctx, int want_phase, const char* who) {
 }
 
 static const char* kNoShardStrands = ": --strand both (RTX_BOTH_STRANDS) is not available in reference-sharded mode";
+static const char* kNoShardBestHits = ": best hits (RTX_OPT_BEST_HITS > 0) are not available in reference-sharded mode";
 
 RTX_API int rtx_shard_phase1(rtx_ctx* ctx) {
     if (ctx && ctx->has_batch && (ctx->bv.flags & RTX_BOTH_STRANDS))
         return set_err(ctx, RTX_ERR_UNSUPPORTED, std::string("rtx_shard_phase1") + kNoShardStrands);
+    if (ctx && ctx->has_batch && ctx->best_hits)
+        return set_err(ctx, RTX_ERR_UNSUPPORTED, std::string("rtx_shard_phase1") + kNoShardBestHits);
     int rc = shard_precheck(ctx, 0, "rtx_shard_phase1");
     if (rc) return rc;
     BatchView& bv = ctx->bv;
@@ -1729,6 +1783,8 @@ static int comm_precheck(rtx_ctx* ctx, const char* who) {
 RTX_API int rtx_shard_run(rtx_ctx* ctx) {
     if (ctx && ctx->has_batch && (ctx->bv.flags & RTX_BOTH_STRANDS))
         return set_err(ctx, RTX_ERR_UNSUPPORTED, std::string("rtx_shard_run") + kNoShardStrands);
+    if (ctx && ctx->has_batch && ctx->best_hits)
+        return set_err(ctx, RTX_ERR_UNSUPPORTED, std::string("rtx_shard_run") + kNoShardBestHits);
     int rc = comm_precheck(ctx, "rtx_shard_run");
     if (rc) return rc;
     CU(cudaSetDevice(ctx->device));
@@ -1970,6 +2026,7 @@ RTX_API int rtx_shard_classify(rtx_ctx* ctx, const rtx_batch* batch, rtx_results
     if (!ctx) return RTX_ERR_INVALID;
     REQUIRE(results != nullptr, "results is NULL");
     if (batch && (batch->flags & RTX_BOTH_STRANDS)) return set_err(ctx, RTX_ERR_UNSUPPORTED, std::string("rtx_shard_classify") + kNoShardStrands);
+    if (ctx->best_hits_opt) return set_err(ctx, RTX_ERR_UNSUPPORTED, std::string("rtx_shard_classify") + kNoShardBestHits);
     int rc = rtx_batch_upload(ctx, batch);
     if (rc == RTX_OK) rc = rtx_shard_run(ctx);
     if (rc == RTX_OK) rc = rtx_shard_gather(ctx, root);

@@ -3,8 +3,9 @@
 // Mirrors the reference's CLI surface, output files and restart behaviour (src/io.rs:112-300, src/main.rs:14-173):
 //   raxtax -d <db.fasta[.gz] | db.bin> -i <queries.fasta[.gz]> [-o PREFIX] [--skip-exact-matches] [--raw-confidence] [--tsv]
 //          [--redo] [--only-db] [--skip-db] [-c] [-t N] [--pin] [-v|-q] [--gpu N] [--gpus N [--shard-references]] [--batch N]
-//          [--strand plus|both]
-// writes <PREFIX>/raxtax.out, raxtax.log, raxtax.ckp, raxtax.json and (with --tsv) raxtax.tsv in the reference's formats
+//          [--strand plus|both] [--best-hits N]
+// writes <PREFIX>/raxtax.out, raxtax.log, raxtax.ckp, raxtax.json, (with --tsv) raxtax.tsv in the reference's formats and (with
+// --best-hits) raxtax.hits, each query's N references with the most shared 8-mers
 // (lineage.rs:17-48), and <PREFIX>/<database stem>.bin, the bincode database of tree.rs:146-164, unless --skip-db.
 // A database path that deserialises as such a .bin is loaded instead of parsed (parser.rs:37-44).  An interrupted run is
 // continued from raxtax.json + raxtax.ckp (io.rs:47-90,156-230) when the flags and the database fingerprint still match.
@@ -38,6 +39,7 @@ struct Args {
     bool skip_exact_matches = false, tsv = false, only_db = false, skip_db = false, clean = false, raw_confidence = false, redo = false,
          pin = false, shard_refs = false, both_strands = false;
     int threads = 0, verbosity = 3 /* Info */, gpu = 0, gpus = 1;
+    unsigned best_hits = 0;  // --best-hits: 0 = no raxtax.hits
     size_t batch = 0;
 };
 
@@ -65,12 +67,14 @@ void usage() {
             "      --batch <N>                      Queries per device batch [default: all]\n"
             "      --strand <STRAND>                plus: classify the queries as given; both: in the orientation that shares more\n"
             "                                       8-mers with some reference, strand column +/- in the outputs [default: plus]\n"
+            "      --best-hits <N>                  Write each query's N (1..64) references with the most shared 8-mers to\n"
+            "                                       raxtax.hits: label, rank, lineage, shared 8-mers, K, reference id\n"
             "  -v, --verbose...                     Increase logging verbosity (repeatable: -vv)\n"
             "  -q, --quiet...                       Decrease logging verbosity (repeatable: -qq)\n");
 }
 
 struct Writers {
-    FILE *primary = nullptr, *tsv = nullptr, *log = nullptr, *progress = nullptr;
+    FILE *primary = nullptr, *tsv = nullptr, *log = nullptr, *progress = nullptr, *hits = nullptr;
     int verbosity = 3;
     std::string pending_labels;  // labels whose result lines are written but possibly still in a stdio buffer
     size_t pending_n = 0;
@@ -82,7 +86,7 @@ struct Writers {
     // (lines of queries not yet listed are what check_incomplete_output removes on resume).
     bool commit() {
         if (pending_n == 0) return !failed;
-        if ((tsv && fflush(tsv) != 0) || fflush(primary) != 0) failed = true;
+        if ((tsv && fflush(tsv) != 0) || (hits && fflush(hits) != 0) || fflush(primary) != 0) failed = true;
         if (!failed && (fwrite(pending_labels.data(), 1, pending_labels.size(), progress) != pending_labels.size() || fflush(progress) != 0)) failed = true;
         pending_labels.clear();
         pending_n = 0;
@@ -97,6 +101,12 @@ int send_cb(void* user, const char* label, const char* primary, const char* tsv)
     w->pending_labels += label;
     w->pending_labels += '\n';
     if (++w->pending_n >= 256 && !w->commit()) return 1;
+    return 0;
+}
+
+int hits_cb(void* user, const char* /*label*/, const char* lines) {  // called right before send_cb of the same query
+    Writers* w = (Writers*)user;
+    if (*lines && (fputs(lines, w->hits) < 0 || fputc('\n', w->hits) == EOF)) return 1;
     return 0;
 }
 
@@ -173,6 +183,7 @@ struct Checkpoint {
     Fingerprint db;
     bool raw_confidence = false, skip_exact_matches = false, tsv = false;
     bool both_strands = false;  // "strand": "both", written only in that mode (a plain run keeps the reference's key set)
+    unsigned best_hits = 0;     // "best_hits": N, written only with --best-hits
     std::set<std::string> processed;  // #[serde(skip)]
 };
 std::string json_escape(const std::string& s) {
@@ -200,10 +211,11 @@ bool checkpoint_save(const Checkpoint& c) {  // Checkpoint::save (io.rs:72-78): 
     if (!f) return false;
     fprintf(f,
             "{\n  \"checkpoint_file\": \"%s\",\n  \"progress_file\": \"%s\",\n  \"db_fingerprint\": {\n    \"path\": \"%s\",\n"
-            "    \"size\": %llu,\n    \"modified\": %llu\n  },\n  \"raw_confidence\": %s,\n  \"skip_exact_matches\": %s,\n  \"tsv\": %s%s\n}",
+            "    \"size\": %llu,\n    \"modified\": %llu\n  },\n  \"raw_confidence\": %s,\n  \"skip_exact_matches\": %s,\n  \"tsv\": %s%s%s\n}",
             json_escape(c.checkpoint_file).c_str(), json_escape(c.progress_file).c_str(), json_escape(c.db.path).c_str(), c.db.size,
             c.db.modified, c.raw_confidence ? "true" : "false", c.skip_exact_matches ? "true" : "false", c.tsv ? "true" : "false",
-            c.both_strands ? ",\n  \"strand\": \"both\"" : "");
+            c.both_strands ? ",\n  \"strand\": \"both\"" : "",
+            c.best_hits ? (",\n  \"best_hits\": " + std::to_string(c.best_hits)).c_str() : "");
     if (fclose(f) != 0) return false;
     return rename(tmp.c_str(), c.checkpoint_file.c_str()) == 0;
 }
@@ -282,6 +294,7 @@ bool checkpoint_load(const std::string& path, Checkpoint* c) {  // serde_json::f
     if (!json_find(j, "modified", &v)) return false;
     c->db.modified = strtoull(v.c_str(), nullptr, 10);
     c->both_strands = json_find(j, "strand", &v) && v == "both";
+    c->best_hits = json_find(j, "best_hits", &v) ? (unsigned)strtoul(v.c_str(), nullptr, 10) : 0u;
     return b("raw_confidence", &c->raw_confidence) && b("skip_exact_matches", &c->skip_exact_matches) && b("tsv", &c->tsv);
 }
 // io::check_incomplete_output (io.rs:156-188): drop the result lines of queries the progress file does not list
@@ -345,6 +358,16 @@ int main(int argc, char** argv) {
             }
             a.both_strands = v == "both";
         }
+        else if (s == "--best-hits") {
+            const std::string v = val("--best-hits");
+            const bool digits = !v.empty() && v.size() <= 2 && v.find_first_not_of("0123456789") == std::string::npos;
+            const unsigned n = digits ? (unsigned)atoi(v.c_str()) : 0u;
+            if (n < 1 || n > 64) {
+                fprintf(stderr, "error: invalid value '%s' for '--best-hits <N>': a number in 1..64 is required\n", v.c_str());
+                return EX_USAGE_;
+            }
+            a.best_hits = n;
+        }
         else if (s == "--verbose") a.verbosity = std::min(5, a.verbosity + 1);  // clap_verbosity_flag::Verbosity<InfoLevel> (io.rs:152-153)
         else if (s == "--quiet") a.verbosity = std::max(0, a.verbosity - 1);
         else if (s.size() >= 2 && s[0] == '-' && s.find_first_not_of('v', 1) == std::string::npos) a.verbosity = std::min(5, a.verbosity + (int)s.size() - 1);  // -v, -vv, ...
@@ -370,8 +393,13 @@ int main(int argc, char** argv) {
         fprintf(stderr, "error: the argument '--strand both' cannot be used with '--shard-references'\n");
         return EX_USAGE_;
     }
+    if (a.best_hits && a.shard_refs) {
+        fprintf(stderr, "error: the argument '--best-hits' cannot be used with '--shard-references'\n");
+        return EX_USAGE_;
+    }
     // ---- Args::get_output (io.rs:202-263): checkpoint, output folder, writers ----------------------------------------
-    const std::string ckp_path = a.prefix + "/raxtax.json", out_path = a.prefix + "/raxtax.out", tsv_path = a.prefix + "/raxtax.tsv";
+    const std::string ckp_path = a.prefix + "/raxtax.json", out_path = a.prefix + "/raxtax.out", tsv_path = a.prefix + "/raxtax.tsv",
+                      hits_path = a.prefix + "/raxtax.hits";
     Checkpoint ckp;
     auto checkpoint_new = [&](Checkpoint* c) {  // Checkpoint::new (io.rs:60-70)
         *c = Checkpoint();
@@ -381,6 +409,7 @@ int main(int argc, char** argv) {
         c->skip_exact_matches = a.skip_exact_matches;
         c->tsv = a.tsv;
         c->both_strands = a.both_strands;
+        c->best_hits = a.best_hits;
         return fingerprint(a.database_path, &c->db);
     };
     bool resumed = false;
@@ -389,12 +418,14 @@ int main(int argc, char** argv) {
         if (checkpoint_load(ckp_path, &old)) {
             Fingerprint now;
             const bool valid = fingerprint(old.db.path, &now) && a.tsv == old.tsv && a.raw_confidence == old.raw_confidence &&
-                               a.skip_exact_matches == old.skip_exact_matches && a.both_strands == old.both_strands && now == old.db;  // checkpoint_valid (io.rs:288-303)
+                               a.skip_exact_matches == old.skip_exact_matches && a.both_strands == old.both_strands && a.best_hits == old.best_hits &&
+                               now == old.db;  // checkpoint_valid (io.rs:288-303)
             if (valid) {
                 std::ifstream prog(old.progress_file);
                 std::string line;
                 while (std::getline(prog, line)) old.processed.insert(line);
-                if (!check_incomplete_output(out_path, old.processed) || (a.tsv && !check_incomplete_output(tsv_path, old.processed))) {
+                if (!check_incomplete_output(out_path, old.processed) || (a.tsv && !check_incomplete_output(tsv_path, old.processed)) ||
+                    (a.best_hits && is_file(hits_path) && !check_incomplete_output(hits_path, old.processed))) {
                     fprintf(stderr, "\x1b[31m[ERROR]\x1b[0m cannot repair the output files under %s\n", a.prefix.c_str());
                     return EX_CANTCREAT_;
                 }
@@ -427,6 +458,7 @@ int main(int argc, char** argv) {
     Writers w;
     w.verbosity = a.verbosity;
     if (a.tsv) w.tsv = fopen(tsv_path.c_str(), mode);
+    if (a.best_hits) w.hits = fopen(hits_path.c_str(), mode);
     w.log = fopen((a.prefix + "/raxtax.log").c_str(), mode);
     if (w.log && restart_note) {
         fprintf(w.log, "[INFO ] Restarting from checkpoint %s\n", ckp.checkpoint_file.c_str());
@@ -434,7 +466,7 @@ int main(int argc, char** argv) {
     }
     w.primary = fopen(out_path.c_str(), mode);
     w.progress = fopen((a.prefix + "/raxtax.ckp").c_str(), mode);
-    if (!w.primary || !w.log || !w.progress || (a.tsv && !w.tsv)) {
+    if (!w.primary || !w.log || !w.progress || (a.tsv && !w.tsv) || (a.best_hits && !w.hits)) {
         fprintf(stderr, "\x1b[31m[ERROR]\x1b[0m cannot create output files under %s\n", a.prefix.c_str());
         return EX_CANTCREAT_;
     }
@@ -529,6 +561,8 @@ int main(int argc, char** argv) {
     auto t0 = std::chrono::steady_clock::now();
     int rc = sharded ? rxh_raxtax_sharded(ctxs.data(), ctxs.size(), queries, tree, a.skip_exact_matches, a.raw_confidence, a.batch, send_cb, &w,
                                           a.tsv, log_cb, &w, &warnings)
+                     : a.best_hits ? rxh_raxtax_best_hits(ctxs.data(), ctxs.size(), queries, tree, a.skip_exact_matches, a.raw_confidence, a.batch,
+                                                          send_cb, &w, a.tsv, log_cb, &w, &warnings, a.both_strands, a.best_hits, hits_cb, &w)
                      : (a.both_strands ? rxh_raxtax_both_strands : rxh_raxtax_multi)(ctxs.data(), ctxs.size(), queries, tree, a.skip_exact_matches,
                                                                                      a.raw_confidence, a.batch, send_cb, &w, a.tsv, log_cb, &w, &warnings);
     double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
@@ -546,7 +580,7 @@ int main(int argc, char** argv) {
         fprintf(w.log, "[INFO ] raxtax(), Elapsed=%.6fs\n", secs);
         fprintf(w.log, "[INFO ] Total Runtime, Elapsed=%.6fs\n", std::chrono::duration<double>(std::chrono::steady_clock::now() - t_total).count());
     }
-    for (FILE* f : {w.primary, w.tsv, w.log, w.progress})
+    for (FILE* f : {w.primary, w.tsv, w.log, w.progress, w.hits})
         if (f) fclose(f);
     if (a.clean) {  // Checkpoint::cleanup (io.rs:80-89); the database only if it lives under PREFIX as <stem>.bin (see the header)
         if (a.verbosity >= 3) fprintf(stderr, "[INFO ] Removing checkpoint files...\n");

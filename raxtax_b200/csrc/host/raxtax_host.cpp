@@ -1555,6 +1555,11 @@ static inline void strand_column(CharBuf& s, bool minus) {
     s.put('\t');
     s.put(minus ? '-' : '+');
 }
+static inline void uint_column(CharBuf& s, u64 v) {
+    s.put('\t');
+    char* p = s.reserve(24);
+    s.n += (size_t)(put_uint(p, v) - p);
+}
 
 static void output_line(CharBuf& s, const std::string& label, const ResultView& r) {  // lineage.rs:17-30
     s.put(label.data(), label.size());
@@ -1654,6 +1659,8 @@ struct ChunkJob {
     std::vector<u64> u_off, uniq_hash;
     std::vector<u8> u_codes;
     std::vector<u8> rc_seq, strand;  // --strand both: a reverse complement being looked up; per distinct sequence, 1 = classified as rc
+    std::vector<u32> hit_n, hit_ref;   // best hits (rtx_batch_best_hits) per distinct sequence
+    std::vector<u16> hit_count;
     PinnedArr<u16> n_kmers;
     PinnedArr<u32> result_begin, first_ref;
     PinnedArr<double> global, conf, local;
@@ -1753,7 +1760,7 @@ struct Worker {
     // emitter's helpers
     struct FormatPart {
         CharBuf buf;
-        std::vector<size_t> off;  // per query: start of the primary string, start of the tsv string (both NUL-terminated)
+        std::vector<size_t> off;  // per query: start of the primary string, of the tsv string and (with best hits) of the hit lines
     };
     std::vector<FormatPart> parts{};
     std::vector<std::thread> helpers{};
@@ -1775,6 +1782,9 @@ struct Worker {
     std::chrono::steady_clock::time_point t_start{}, t_first_issue{}, t_last_collect{};
     std::atomic<bool> first_issued{false};
     bool both = false;  // --strand both (rxh_raxtax_both_strands): RTX_BOTH_STRANDS batches, strand column in both outputs
+    u32 best_hits = 0;  // --best-hits (rxh_raxtax_best_hits): RTX_OPT_BEST_HITS of every batch, lines to hits_sender
+    rxh_hits_sender hits_sender = nullptr;
+    void* hits_user = nullptr;
     static std::chrono::steady_clock::time_point now() { return std::chrono::steady_clock::now(); }
 
     void fail(const std::string& what) {
@@ -1916,6 +1926,8 @@ struct Worker {
         batch.flags = (skip_exact_matches ? RTX_SKIP_EXACT_MATCHES : 0u) | (raw_confidence ? RTX_RAW_CONFIDENCE : 0u) | (both ? RTX_BOTH_STRANDS : 0u);
         j.dev_slot = dev_slot;
         if (rtx_batch_slot(ctx, dev_slot)) throw Error(std::string("rtx_batch_slot: ") + rtx_last_error(ctx));
+        if (best_hits && rtx_ctx_set_option(ctx, RTX_OPT_BEST_HITS, best_hits))
+            throw Error(std::string("rtx_ctx_set_option(RTX_OPT_BEST_HITS): ") + rtx_last_error(ctx));
         int rc = rtx_batch_upload(ctx, &batch);
         if (rc == RTX_ERR_CUDA && is_oom(ctx)) return false;
         if (rc) throw Error(std::string("rtx_batch_upload: ") + rtx_last_error(ctx));
@@ -1962,6 +1974,13 @@ struct Worker {
             j.strand.resize(std::max<size_t>(j.n_uniq, 1));
             if (rtx_batch_strands(ctx, j.strand.data())) throw Error(std::string("rtx_batch_strands: ") + rtx_last_error(ctx));
             log_exact(j);
+        }
+        if (best_hits) {
+            j.hit_n.resize(std::max<size_t>(j.n_uniq, 1));
+            j.hit_ref.resize(std::max<size_t>(j.n_uniq, 1) * best_hits);
+            j.hit_count.resize(std::max<size_t>(j.n_uniq, 1) * best_hits);
+            if (rtx_batch_best_hits(ctx, j.hit_n.data(), j.hit_ref.data(), j.hit_count.data()))
+                throw Error(std::string("rtx_batch_best_hits: ") + rtx_last_error(ctx));
         }
     }
 
@@ -2158,6 +2177,24 @@ struct Worker {
                 }
                 out.buf.put('\0');
             }
+            if (hits_sender) {  // {label}\t{rank}\t{lineage}\t{shared 8-mers}\t{K}\t{reference id}[\t{strand}]
+                out.off.push_back(out.buf.n);
+                const std::string& label = qs.labels[q];
+                for (u32 k = 0; k < j.hit_n[u]; ++k) {
+                    const size_t h = (size_t)u * best_hits + k;
+                    const u32 ref = j.hit_ref[h];
+                    if (k) out.buf.put('\n');
+                    out.buf.put(label.data(), label.size());
+                    uint_column(out.buf, k + 1);
+                    out.buf.put('\t');
+                    out.buf.put(tree.lineages[ref].data(), tree.lineages[ref].size());
+                    uint_column(out.buf, j.hit_count[h]);
+                    uint_column(out.buf, j.n_kmers.p[u]);
+                    uint_column(out.buf, ref);
+                    if (both) strand_column(out.buf, minus);
+                }
+                out.buf.put('\0');
+            }
         }
     }
     static void part_range(size_t cn, size_t n_parts, size_t k, size_t* i0, size_t* i1) {
@@ -2217,9 +2254,13 @@ struct Worker {
             part_range(j.cn, n_parts, k, &i0, &i1);
             const FormatPart& fp = parts[k];
             const char* base = fp.buf.v.data();
+            const size_t stride = hits_sender ? 3 : 2;
             for (size_t i = i0; i < i1; ++i) {
-                const size_t o = (i - i0) * 2;
-                if (sender(sender_user, qs.labels[j.c0 + i].c_str(), base + fp.off[o], tsv ? base + fp.off[o + 1] : nullptr) != 0)
+                const size_t o = (i - i0) * stride;
+                const char* label = qs.labels[j.c0 + i].c_str();
+                if (hits_sender && hits_sender(hits_user, label, base + fp.off[o + 2]) != 0)
+                    throw Error("sending on a disconnected channel (best hits)");
+                if (sender(sender_user, label, base + fp.off[o], tsv ? base + fp.off[o + 1] : nullptr) != 0)
                     throw Error("sending on a disconnected channel (raxtax.rs:87)");
             }
         }
@@ -2335,10 +2376,15 @@ RXH_API size_t rxh_plan_chunks(size_t n_queries, size_t n_ctx, size_t chunk_size
 
 static int raxtax_query_partitioned(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queries* queries, const rxh_tree* tree_h, int skip_exact_matches,
                                     int raw_confidence, size_t chunk_size, rxh_sender sender, void* sender_user, int tsv, rxh_logger logger,
-                                    void* logger_user, int* warnings, int both_strands, const char* who) {
+                                    void* logger_user, int* warnings, int both_strands, u32 best_hits, rxh_hits_sender hits_sender,
+                                    void* hits_user, const char* who) {
     if (warnings) *warnings = 0;
     if (!ctxs || n_ctx == 0 || !queries || !tree_h) {
         g_err = std::string(who) + ": no context";
+        return -1;
+    }
+    if (best_hits > 64) {
+        g_err = std::string(who) + ": best_hits must be in [0, 64]";
         return -1;
     }
     const size_t nq = queries->q->size();
@@ -2347,7 +2393,12 @@ static int raxtax_query_partitioned(rtx_ctx* const* ctxs, size_t n_ctx, const rx
     Worker w{*tree_h->t, *queries->q, nq, chunk_size, skip_exact_matches, raw_confidence, tsv, sender, sender_user, logger, logger_user};
     w.ramp = ramp;
     w.both = both_strands != 0;
+    w.best_hits = best_hits;
+    w.hits_sender = best_hits ? hits_sender : nullptr;
+    w.hits_user = hits_user;
     w.run(ctxs, n_ctx);
+    if (best_hits)  // the option outlives the call in the contexts: leave them as they were handed in
+        for (size_t i = 0; i < n_ctx; ++i) rtx_ctx_set_option(ctxs[i], RTX_OPT_BEST_HITS, 0);
     if (warnings) *warnings = w.warned.load() ? 1 : 0;
     if (w.failed.load()) {
         g_err = w.err;
@@ -2360,14 +2411,22 @@ RXH_API int rxh_raxtax_multi(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queri
                              int raw_confidence, size_t chunk_size, rxh_sender sender, void* sender_user, int tsv, rxh_logger logger,
                              void* logger_user, int* warnings) {
     return raxtax_query_partitioned(ctxs, n_ctx, queries, tree_h, skip_exact_matches, raw_confidence, chunk_size, sender, sender_user, tsv, logger,
-                                    logger_user, warnings, 0, "rxh_raxtax_multi");
+                                    logger_user, warnings, 0, 0, nullptr, nullptr, "rxh_raxtax_multi");
 }
 
 RXH_API int rxh_raxtax_both_strands(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queries* queries, const rxh_tree* tree_h, int skip_exact_matches,
                                     int raw_confidence, size_t chunk_size, rxh_sender sender, void* sender_user, int tsv, rxh_logger logger,
                                     void* logger_user, int* warnings) {
     return raxtax_query_partitioned(ctxs, n_ctx, queries, tree_h, skip_exact_matches, raw_confidence, chunk_size, sender, sender_user, tsv, logger,
-                                    logger_user, warnings, 1, "rxh_raxtax_both_strands");
+                                    logger_user, warnings, 1, 0, nullptr, nullptr, "rxh_raxtax_both_strands");
+}
+
+RXH_API int rxh_raxtax_best_hits(rtx_ctx* const* ctxs, size_t n_ctx, const rxh_queries* queries, const rxh_tree* tree_h, int skip_exact_matches,
+                                 int raw_confidence, size_t chunk_size, rxh_sender sender, void* sender_user, int tsv, rxh_logger logger,
+                                 void* logger_user, int* warnings, int both_strands, uint32_t best_hits, rxh_hits_sender hits_sender,
+                                 void* hits_user) {
+    return raxtax_query_partitioned(ctxs, n_ctx, queries, tree_h, skip_exact_matches, raw_confidence, chunk_size, sender, sender_user, tsv, logger,
+                                    logger_user, warnings, both_strands, best_hits, hits_sender, hits_user, "rxh_raxtax_best_hits");
 }
 
 // Reference-sharded mode: the result lines the ranks emitted for one batch, merged per query.  Lines are ordered like
